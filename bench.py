@@ -4,7 +4,7 @@ path, BASELINE.json north_star) on synthetic EndoVis18-shaped clips, plus the pi
 loss step (the second hot path) timed beside it.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                  [--config seg|cadis|finetune_sgd|pretrain]
+                  [--config seg|cadis|finetune_sgd|pretrain] [--dump-outputs DIR]
 
 Default (``--config seg`` = configs[1] of BASELINE.json: batch 8, bf16, 1 B200): a step = forward +
 backward + optimizer step of ``SwinTransformerLayerv5`` (dim 512, 64x80 tokens, 4 heads, 12 blocks +
@@ -86,7 +86,13 @@ def parse():
                          "step; 'ddp' = torch DistributedDataParallel, eager steps")
     ap.add_argument("--wire", default="bf16", choices=["fp32", "bf16"], help="--dp flat: dtype of the gradients on the wire")
     ap.add_argument("--segments", type=int, default=4, help="--dp flat: graph segments of the backward (1 = one all-reduce)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last of them computed as DIR/<name>.npy (float32): the loss, "
+                         "the head's two outputs, every parameter and its gradient (a fixed seeded sample of the large ones, "
+                         "64 MB at most), so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the GPU path (--impl ours)")
     if args.clips <= 0:
         args.clips = CONFIGS[args.config][1]
     return args
@@ -151,6 +157,49 @@ class ClockSampler:
         if sm:
             out.update(sm_mhz=statistics.median(sm), sm_max_mhz=max(mx), reasons=sorted(reasons), samples=len(sm))
         return out
+
+
+DUMP_BYTES = 64 << 20          # --dump-outputs: the whole dump
+DUMP_OUTPUT_CAP = 1 << 22      # elements kept of the loss / head outputs
+DUMP_PARAM_CAP = 1 << 14       # elements kept of each parameter, gradient and key-encoder parameter
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each (name, tensor, cap) as ``out_dir/<name>.npy`` in float32: the whole tensor when it has at most ``cap``
+    elements, else ``cap`` of them at positions drawn from a generator seeded by the name (the same positions on every
+    run and every build, for a tensor of the same size)."""
+    import zlib
+    import numpy as np
+    import torch
+    nbytes = sum(4 * min(t.numel(), cap) for _, t, cap in arrays)
+    if nbytes > DUMP_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs would write {nbytes} bytes, more than {DUMP_BYTES}")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t, cap in arrays:
+        t = t.detach()
+        if t.numel() > cap:
+            gen = torch.Generator().manual_seed(zlib.crc32(name.encode()))
+            idx = torch.randint(0, t.numel(), (cap,), generator=gen).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+    print(f"bench.py: wrote {len(arrays)} arrays ({nbytes / 2 ** 20:.1f} MB) to {out_dir}", file=sys.stderr)
+
+
+def reset_training_state(params, initial, opt):
+    """Put ``params`` back to ``initial`` and ``opt`` back to its state before its first step, in place (a captured step
+    graph reads these very tensors).  Every state tensor of FusedAdam, SGD and LARS -- moments, momentum buffers, Adam's
+    device step count -- is zero before the first step.  The bf16 weight shadows are rewritten from the weights."""
+    import torch
+    from stswincl_b200 import optim as soptim
+    with torch.no_grad():
+        for p, v in zip(params, initial):
+            p.copy_(v)
+        for t in [v for st in opt.state.values() for v in st.values()] + [v for g in opt.param_groups for v in g.values()]:
+            if torch.is_tensor(t):
+                t.zero_()
+    for p in params:
+        if getattr(p, "_stswin_shadow", None) is not None:
+            soptim.bf16_weight(p)
 
 
 def workload_config(name, clips, graph=None, extra=None):
@@ -356,6 +405,8 @@ def run_ours(args):
     from stswincl_b200 import dist as sdist
     if world > 1:
         sdist.broadcast_parameters(params)                 # replicas start identical (DDP's constructor does the same)
+    state_params = params + (list(key_model.parameters()) if key_model is not None else [])
+    initial = [p.detach().clone() for p in state_params] if args.dump_outputs else None
     if opt_kind == "adam":
         opt = soptim.FusedAdam(model.parameters(), lr=3e-5)
     elif opt_kind == "sgd":
@@ -382,10 +433,20 @@ def run_ours(args):
         up = torch.nn.functional.interpolate(y2[:, -1, :256], size=y1.shape[-2:], mode="nearest")
         return y1[:, -1, :256] + up
 
+    kept = {}
+
+    def keep(loss, y1, y2):
+        # --dump-outputs: hold the step's loss and head outputs (a captured graph rewrites these tensors on every replay).
+        # Detached: a reference to the autograd graph would keep its AccumulateGrad nodes alive into the next step, whose
+        # stream mismatch breaks the graph capture.
+        if args.dump_outputs:
+            kept.update(loss=loss.detach(), y1=y1.detach(), y2=y2.detach())
+        return loss
+
     def forward_loss(x):
         if not pretrain:
             y1, y2 = net(x)
-            return torch.sum(y1 * g1, dtype=torch.float32) + torch.sum(y2 * g2, dtype=torch.float32)
+            return keep(torch.sum(y1 * g1, dtype=torch.float32) + torch.sum(y2 * g2, dtype=torch.float32), y1, y2)
         # PixPro.forward (PixPro_swin_v5.py:291-561) on the Swin head: two query passes, EMA, six no-grad key passes
         y1, y2 = net(x[:2 * B])
         pred_1, pred_2 = embed(y1[:B], y2[:B]), embed(y1[B:], y2[B:])
@@ -393,7 +454,8 @@ def run_ours(args):
             soptim.momentum_update(list(model.parameters()), list(key_model.parameters()), 0.99)
             k1, k2 = key_model(x)
             keys = [embed(k1[i * B:(i + 1) * B], k2[i * B:(i + 1) * B]) for i in range(6)]
-        return contrast.consistency_loss_tail(pred_1, pred_2, *keys, *masks, K, normalize=True, cross_rank_negatives=world > 1)
+        return keep(contrast.consistency_loss_tail(pred_1, pred_2, *keys, *masks, K, normalize=True, cross_rank_negatives=world > 1),
+                    y1, y2)
 
     def barrier():
         if world > 1:
@@ -422,7 +484,7 @@ def run_ours(args):
     use_graph = not args.no_graph and not (pretrain and world > 1)      # NCCL all-gather inside the loss: eager
     stepper = None
     if flat_dp and not pretrain:
-        stepper = sdist.SegmentedStep(model, opt, lambda y: torch.sum(y[0] * g1, dtype=torch.float32) + torch.sum(y[1] * g2, dtype=torch.float32),
+        stepper = sdist.SegmentedStep(model, opt, lambda y: keep(torch.sum(y[0] * g1, dtype=torch.float32) + torch.sum(y[1] * g2, dtype=torch.float32), *y),
                                       segments=max(1, args.segments), wire_dtype=torch.bfloat16 if args.wire == "bf16" else torch.float32,
                                       use_graph=use_graph)
     flat = sdist.FlatGradients(params) if (flat_dp and stepper is None) else None
@@ -507,9 +569,26 @@ def run_ours(args):
     with ClockSampler(local if rank == 0 else None) as clk:
         for _ in range(12):
             run_step(cur_x())
-        ms_step = timed(lambda i: run_step(cur_x()), args.steps)
+        if args.dump_outputs:
+            # the last timed step starts from the seeded initial weights and a fresh optimizer, so that its inputs are the
+            # same on every run: the steps before it repeat one batch, and Adam turns the reordered fp32 sums of a step into
+            # weight differences that grow from step to step.  The reset itself is not timed.
+            ms_step = timed(lambda i: run_step(cur_x()), args.steps - 1) * (args.steps - 1) if args.steps > 1 else 0.0
+            reset_training_state(state_params, initial, opt)
+            ms_step = (ms_step + timed(lambda i: run_step(cur_x()), 1)) / args.steps
+        else:
+            ms_step = timed(lambda i: run_step(cur_x()), args.steps)
     launches = launches_per_step * args.steps
     clocks = clk.summary()
+    if args.dump_outputs and rank == 0:
+        # with --dp flat the optimizer reads the all-reduced gradients from the stepper's buckets, not from p.grad
+        grad_of = (lambda p: stepper._view_of[id(p)]) if stepper is not None else (lambda p: p.grad)
+        arrays = [(k, kept[k], DUMP_OUTPUT_CAP) for k in ("loss", "y1", "y2")]
+        for n, p in model.named_parameters():
+            arrays += [("param." + n, p, DUMP_PARAM_CAP), ("grad." + n, grad_of(p), DUMP_PARAM_CAP)]
+        if key_model is not None:
+            arrays += [("key_param." + n, p, DUMP_PARAM_CAP) for n, p in key_model.named_parameters()]
+        dump_outputs(args.dump_outputs, arrays)
 
     # ---- end to end: pinned host features -> H2D (copy stream, double buffered) -> step -> loss.item()
     x_host = x_dev.cpu().pin_memory()

@@ -29,6 +29,54 @@ def test_non_zero_ranks_of_the_reference_arm_exit_quietly():
     assert out.returncode == 0 and out.stdout.strip() == ""
 
 
+def test_dump_outputs_writes_float32_and_samples_large_arrays_at_fixed_positions(tmp_path, monkeypatch):
+    import numpy as np
+    import pytest
+    import torch
+    import bench
+    gen = torch.Generator().manual_seed(0)
+    big = torch.randn(40, 50, generator=gen).to(torch.bfloat16)
+    small = torch.randn(7, 5, generator=gen)
+    arrays = [("loss", torch.tensor(1.5), 16), ("param.big", big, 500), ("grad.small", small, 500)]
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays)
+    got = {n: np.load(tmp_path / "a" / (n + ".npy")) for n, _, _ in arrays}
+    for n, a in got.items():
+        assert a.dtype == np.float32 and np.array_equal(a, np.load(tmp_path / "b" / (n + ".npy"))), n
+    assert got["loss"] == 1.5 and np.array_equal(got["grad.small"], small.numpy())
+    assert got["param.big"].shape == (500,) and np.isin(got["param.big"], big.float().numpy()).all()
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4 * 500)
+    with pytest.raises(SystemExit):
+        bench.dump_outputs(str(tmp_path / "c"), arrays)
+    assert not (tmp_path / "c").exists()
+
+
+def test_reset_training_state_makes_the_next_step_a_first_step():
+    import torch
+    import bench
+    x = torch.randn(8, 6, generator=torch.Generator().manual_seed(1))
+    for make_opt in (lambda ps: torch.optim.Adam(ps, lr=1e-2, foreach=False),
+                     lambda ps: torch.optim.SGD(ps, lr=1e-2, momentum=0.9, weight_decay=1e-4, foreach=False)):
+        torch.manual_seed(0)
+        fresh, used = torch.nn.Linear(6, 5), torch.nn.Linear(6, 5)
+        used.load_state_dict(fresh.state_dict())
+        initial = [p.detach().clone() for p in used.parameters()]
+        o_fresh, o_used = make_opt(list(fresh.parameters())), make_opt(list(used.parameters()))
+
+        def step(m, o):
+            o.zero_grad()
+            (m(x) ** 2).sum().backward()
+            o.step()
+
+        for _ in range(3):
+            step(used, o_used)
+        bench.reset_training_state(list(used.parameters()), initial, o_used)
+        assert all(torch.equal(p, q) for p, q in zip(used.parameters(), fresh.parameters()))
+        step(fresh, o_fresh)
+        step(used, o_used)
+        assert all(torch.equal(p, q) for p, q in zip(used.parameters(), fresh.parameters())), make_opt
+
+
 def test_gpu_arm_fails_loudly_without_a_device():
     import torch
     if torch.cuda.is_available():

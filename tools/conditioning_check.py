@@ -1,11 +1,12 @@
 """How sensitive are the layer-golden gradients to bf16 rounding?  Runs the fp32 oracle with the
 block boundaries (and the 2-D weights) rounded to bf16 and prints the deviation from the reference
 golden per quantity.  CPU only."""
-import sys, numpy as np, torch
-sys.path.insert(0,'/root/repo')
+import os, sys, numpy as np, torch
+ROOT=os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0,ROOT)
 from oracle import swin_oracle as so, make_goldens as mg
 c=mg.LAYER_CASE; H,W=c["res"]
-g=np.load('/root/repo/tests/golden/swin_layer.npz')
+g=np.load(os.path.join(ROOT,'tests','golden','swin_layer.npz'))
 params=so.make_layer_params(c["dim"],c["res"],c["heads"],c["seed"])
 def rnd(x): return x + (x.bfloat16().float()-x).detach()
 orig_block=so.swin_block
