@@ -56,7 +56,9 @@ int stswin_set_device(int device);
 #define STSWIN_EPI_BIAS 0          /* D = acc + bias                                  */
 #define STSWIN_EPI_BIAS_RES 1      /* D = acc + bias + aux            (residual add)  */
 #define STSWIN_EPI_BIAS_GELU 2     /* u = acc + bias ; D = gelu_erf(u) ; D2 = gelu_erf'(u) */
-#define STSWIN_EPI_MUL_AUX 3       /* D = acc * aux     (dgrad through GELU: aux = D2)  */
+/* The two x-aux modes add `bias` (when not NULL) before the product: D = (acc + bias) * aux.  The block's dgrad passes
+ * NULL; the term is kept because it is free in the epilogue and is what a Linear followed by an elementwise gate needs. */
+#define STSWIN_EPI_MUL_AUX 3       /* D = (acc + bias) * aux     (dgrad through GELU: aux = D2, bias NULL) */
 #define STSWIN_EPI_F32_REDUCE 4    /* D(fp32) += acc, split-K                          */
 #define STSWIN_EPI_BIAS_GELU_FWD 5 /* D = gelu_erf(acc + bias)      (inference: no D2) */
 /* The derivative is only ever a multiplier of the backward and lies in [-0.13, 1.13]: the two modes below keep it as ONE
@@ -64,7 +66,7 @@ int stswin_set_device(int device);
  * multiples of 16): q = round((gelu'(u) + 0.14) * 255 / 1.28), i.e. a step of 0.005 (|error| <= 0.0025, the bf16 rounding of
  * a value near 1 is 0.002-0.004).  fc1 + GELU writes 1.28 GB per stage-1 launch in the bf16 form and is HBM-write bound. */
 #define STSWIN_EPI_BIAS_GELU_Q8 6  /* D = gelu_erf(acc + bias) ; D2(uint8) = quantised gelu_erf'(acc + bias) */
-#define STSWIN_EPI_MUL_AUX_Q8 7    /* D = acc * dequant(aux)        (aux = the uint8 D2 of mode 6) */
+#define STSWIN_EPI_MUL_AUX_Q8 7    /* D = (acc + bias) * dequant(aux)  (aux = the uint8 D2 of mode 6) */
 
 int stswin_gemm_bf16(const void* A, int a_major, int64_t lda,
                      const void* B, int b_major, int64_t ldb,
