@@ -38,25 +38,18 @@
 
 namespace stswin {
 
-int fill_geom(WinGeom* gm, int B, int T, int H, int W, int C, int nH, int ws, int shift);
-int make_window_tmaps(WinMaps* maps, const void* base, const WinGeom& gm, int channels);
-
 namespace {
 
 constexpr int NRH = 5;                         // ring H: first-pass chunks, streamed from HBM
 constexpr int NRL = 4;                         // ring L: second-pass chunks, re-read from L2
-constexpr int SLOT_BYTES = 128 * 128;
 constexpr int PD_BYTES = 2 * SLOT_BYTES;       // [128 x 128] bf16 as two K-major halves
-constexpr int TAB_MAX = 15 * 15;
 constexpr int NUM_THREADS = 512;               // warpgroup 0: producers H / L, MMA issuer; 1: softmax backward; 2, 3: drain
 constexpr int SMEM_BYTES = 1024 + (NRH + NRL) * SLOT_BYTES + 2 * PD_BYTES + 128 * 4 +
                            4 * (TAB_MAX + 1) * 4 + 256;
-constexpr float kMaskLog2e = -100.0f * 1.4426950408889634f;
 STSWIN_TRACE_DECL(g_trace_bwd)
 
-// L, GEN as in the forward kernel.  WS > 0: fast path for the shipped geometries (compile-time column
-// maps; the bias-table gradient is summed in registers).  ORDER: 0 unshifted (row-major), 2 shifted
-// (quadrant order for the windows that wrap).  SHT: heads per 64-channel group (2 when head_dim is 32).
+// L, WS, ORDER, GEN, LWT as in the forward kernel, with the same instantiations; WS > 0 also sums the
+// bias-table gradient in registers.  SHT: heads per 64-channel group (2 when head_dim is 32).
 template <int L, int WS, int ORDER, int SHT, bool GEN, int LWT>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 winattn_bwd_kernel(const __grid_constant__ WinMaps tm_qkv, const __grid_constant__ WinMaps tm_do,
@@ -487,8 +480,8 @@ winattn_bwd_kernel(const __grid_constant__ WinMaps tm_qkv, const __grid_constant
           }
         };
         // a warp never straddles two windows for L >= 32, so the branch is warp-uniform
-        if (ORDER == 0 || (ORDER == 2 && !rg.wraps)) softmax_bwd_fast(std::false_type{});
-        else                                         softmax_bwd_fast(std::true_type{});
+        if (ORDER == 0 || !rg.wraps) softmax_bwd_fast(std::false_type{});
+        else                         softmax_bwd_fast(std::true_type{});
       } else {
         // ---- generic path: per-column look-up table (any order, dense mask, window tags); the
         //      bias-table gradient goes through the shared bins (no static column -> position map)
@@ -660,12 +653,6 @@ winattn_bwd_kernel(const __grid_constant__ WinMaps tm_qkv, const __grid_constant
   }
 }
 
-template <typename K>
-int set_smem_bwd(K kern, int bytes) {
-  STSWIN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
-  return kOk;
-}
-
 }  // namespace
 
 #ifdef STSWIN_TRACE
@@ -680,65 +667,21 @@ int winattn_bwd(const void* qkv, const float* bias_table, const float* lse2, con
                 float qk_scale, const float* mask, int mask_windows, cudaStream_t stream) {
   STSWIN_CHECK_ARG(qkv && bias_table && lse2 && d_out && d_qkv && d_table, "winattn_bwd: null pointer");
   WinGeom gm;
-  int rc = fill_geom(&gm, B, T, H, W, C, nH, ws, shift);
+  int rc = fill_geom(&gm, B, T, H, W, C, nH, ws, shift, qk_scale, mask, mask_windows);
   if (rc != kOk) return rc;
-  if (qk_scale > 0.f) { gm.scale = qk_scale; gm.scale_log2e = qk_scale * 1.4426950408889634f; }
-  STSWIN_CHECK_ARG(mask == nullptr || mask_windows > 0, "winattn: mask given with mask_windows <= 0");
-  gm.mask = mask; gm.mask_nw = mask_windows;
-  if (gm.shift > 0 && gm.ra != gm.rb) gm.general = 1;     // unequal rectangles: no static column -> position fold
-  gm.perm = (gm.shift > 0 && gm.nWh > 1 && gm.nWw > 1) ? 1 : 0;   // interior windows first: one token-order switch per CTA
   WinMaps tq, td;
   if ((rc = make_window_tmaps(&tq, qkv, gm, 3 * C)) != kOk) return rc;
   if ((rc = make_window_tmaps(&td, d_out, gm, C)) != kOk) return rc;
   STSWIN_CHECK_ARG((reinterpret_cast<uintptr_t>(d_qkv) & 31) == 0, "winattn_bwd: d_qkv must be 32-byte aligned");
-  const int items = gm.num_tiles * gm.ngrp;
-  int grid = items < num_sms() ? items : num_sms();
-  grid -= grid % gm.ngrp;                 // one head group per CTA (items is a multiple of ngrp, so grid >= ngrp)
-  if (grid < gm.ngrp) return set_error(kErrUnsupported, "winattn_bwd: %d head groups exceed the SM count", gm.ngrp);
-#define STSWIN_LAUNCH_BWD(LL, WW, OO, SS, GG, PP)                                                              \
-  {                                                                                                            \
-    if ((rc = set_smem_bwd(winattn_bwd_kernel<LL, WW, OO, SS, GG, PP>, SMEM_BYTES)) != kOk) return rc;         \
-    STSWIN_CUDA(launch_pdl(winattn_bwd_kernel<LL, WW, OO, SS, GG, PP>, dim3(grid), dim3(NUM_THREADS), (size_t)SMEM_BYTES, stream, \
-                           tq, td, static_cast<__nv_bfloat16*>(d_qkv), bias_table, lse2, d_table, d_qkv_colsum, gm)); \
-  }
-#define STSWIN_LAUNCH_BWD_P(LL, WW, OO, GG, PP)                 \
-  {                                                             \
-    if (gm.SH == 1) STSWIN_LAUNCH_BWD(LL, WW, OO, 1, GG, PP)    \
-    else STSWIN_LAUNCH_BWD(LL, WW, OO, 2, GG, PP)               \
-  }
-#define STSWIN_LAUNCH_BWD_S(LL, WW, OO, GG) STSWIN_LAUNCH_BWD_P(LL, WW, OO, GG, LL)
-  // fast path: the shipped geometries (ws 8 or 4, 1 or 2 frames per window, shift 0 or ws/2, no dense mask)
-  const bool fast = !gm.general && mask == nullptr && (shift == 0 || 2 * shift == ws) &&
-                    ((ws == 8 && (gm.L == 128 || gm.L == 64)) || (ws == 4 && gm.L == 32));
-  const bool shifted = shift > 0;
-  // odd windows in padded slots (7x7 and 5x5 with one or two frames), shift 0 or ws/2: compile-time maps as well
-  const bool fastp = mask == nullptr && (shift == 0 || shift == ws / 2) &&
-                     ((ws == 7 && (gm.L == 49 || gm.L == 98)) || (ws == 5 && (gm.L == 25 || gm.L == 50)));
-  if (fastp && ws == 7 && gm.L == 98 && !shifted) STSWIN_LAUNCH_BWD_P(128, 7, 0, false, 98)
-  else if (fastp && ws == 7 && gm.L == 98) STSWIN_LAUNCH_BWD_P(128, 7, 2, false, 98)
-  else if (fastp && ws == 7 && !shifted) STSWIN_LAUNCH_BWD_P(64, 7, 0, false, 49)
-  else if (fastp && ws == 7) STSWIN_LAUNCH_BWD_P(64, 7, 2, false, 49)
-  else if (fastp && gm.L == 50 && !shifted) STSWIN_LAUNCH_BWD_P(64, 5, 0, false, 50)
-  else if (fastp && gm.L == 50) STSWIN_LAUNCH_BWD_P(64, 5, 2, false, 50)
-  else if (fastp && !shifted) STSWIN_LAUNCH_BWD_P(32, 5, 0, false, 25)
-  else if (fastp) STSWIN_LAUNCH_BWD_P(32, 5, 2, false, 25)
-  else if (gm.general && gm.slot <= 8 && 32 % gm.slot == 0) STSWIN_LAUNCH_BWD_S(32, 0, 0, true)   // windows of 4 / 8 tokens
-  else if (gm.general) STSWIN_LAUNCH_BWD_S(128, 0, 0, true)
-  else if (fast && gm.L == 128 && !shifted) STSWIN_LAUNCH_BWD_S(128, 8, 0, false)
-  else if (fast && gm.L == 128) STSWIN_LAUNCH_BWD_S(128, 8, 2, false)
-  else if (fast && gm.L == 64 && !shifted) STSWIN_LAUNCH_BWD_S(64, 8, 0, false)
-  else if (fast && gm.L == 64) STSWIN_LAUNCH_BWD_S(64, 8, 2, false)
-  else if (fast && gm.L == 32 && !shifted) STSWIN_LAUNCH_BWD_S(32, 4, 0, false)
-  else if (fast && gm.L == 32) STSWIN_LAUNCH_BWD_S(32, 4, 2, false)
-  else if (gm.L == 16) STSWIN_LAUNCH_BWD_S(16, 0, 0, false)
-  else if (gm.L == 32) STSWIN_LAUNCH_BWD_S(32, 0, 0, false)
-  else if (gm.L == 64) STSWIN_LAUNCH_BWD_S(64, 0, 0, false)
-  else STSWIN_LAUNCH_BWD_S(128, 0, 0, false)
-#undef STSWIN_LAUNCH_BWD_P
-#undef STSWIN_LAUNCH_BWD_S
-#undef STSWIN_LAUNCH_BWD
-  STSWIN_CUDA(cudaGetLastError());
-  return kOk;
+  return dispatch_variant(select_variant(gm, true), [&](auto v) {
+    using V = decltype(v);
+    auto launch = [&](auto kern) {
+      return launch_winattn(kern, gm, NUM_THREADS, SMEM_BYTES, stream, tq, td, static_cast<__nv_bfloat16*>(d_qkv),
+                            bias_table, lse2, d_table, d_qkv_colsum, gm);
+    };
+    if (gm.SH == 1) return launch(winattn_bwd_kernel<V::L, V::WS, V::ORDER, 1, V::GEN, V::LWT>);
+    return launch(winattn_bwd_kernel<V::L, V::WS, V::ORDER, 2, V::GEN, V::LWT>);
+  });
 }
 
 }  // namespace stswin

@@ -16,8 +16,13 @@
 #pragma once
 
 #include "common.cuh"
+#include "host_util.h"
 
 namespace stswin {
+
+constexpr int SLOT_BYTES = 128 * 128;          // one operand chunk: 128 rows x 64 bf16
+constexpr int TAB_MAX = 15 * 15;               // (2*ws-1)^2 for ws <= 8
+constexpr float kMaskLog2e = -100.0f * 1.4426950408889634f;
 
 // Timeline tracing for tools/trace_attn.py (debug builds with -DSTSWIN_TRACE only): CTA 0 records
 // clock64() at named points of its first 64 work items.
@@ -36,7 +41,6 @@ struct WinGeom {
   int B, T, H, W, C, nH, ws, shift;
   int hd, N, L, G, nWh, nWw, nW, total_windows, num_tiles, nc;   // nc = 64-channel chunks per head group
   int slot;           // tile rows from one window of the tile to the next (>= L, see above)
-  int lag;            // forward: the S product of unit u+1 is issued before the P V product of unit u
   int SH, ngrp, gch;   // head_dim >= 64: SH = 1, a "head group" is one head (gch = hd channels).
                        // head_dim 32  : SH = 2 heads share one 64-channel chunk (gch = 64); S / dP use
                        // the head's 32-channel K sub-range of the chunk, the output products run over
@@ -45,13 +49,13 @@ struct WinGeom {
   float scale;                                                    // hd^-0.5
   int ra, rb;         // a shifted window that wraps is moved as 2x2 rectangles of (ws-shift | shift) rows x columns
   int roff[5];        // first tile row of rectangle k inside its window's L rows (roff[4] = L)
-  int general;        // 1: L is not 16/32/64/128 -> the look-up-table kernels run their "whole row + window tag" path
+  int general;        // 1: L is not 16/32/64/128, or (backward) a shift with unequal rectangles: see select_variant
   const float* mask;  // optional dense additive mask [mask_nw, N, N] (WindowAttention.forward's `mask`
   int mask_nw;        //   argument, swin_512.py:127-131), applied ON TOP of the closed-form shift mask; or null
   unsigned long long mg_nW, mg_nWw;   // ceil(2^32 / nW), ceil(2^32 / nWw): exact division of window indices by multiply-shift
-  int perm;           // 1: window indices are enumerated interior-windows-first (see window_coords)
-  int uniform_quad;   // 1: every window of a shifted block is moved as four quadrant boxes (one token
-                      //    order per launch; the backward kernel needs that to sum dS across tiles)
+  int perm;           // 1 (backward, shifted): window indices are enumerated interior-windows-first (see window_coords)
+  int uniform_quad;   // always 0: only the windows that wrap use quadrant order.  Kept with quad_order(): without this
+                      //   run-time select, ptxas spills the backward kernel's head group in winattn_bwd_kernel<32,4,2,1,...>
 };
 
 struct RowGeom {
@@ -207,9 +211,10 @@ __device__ __forceinline__ int fast_div(int n, unsigned long long mg) {
 }
 
 // row_geom for the fast-path geometries: slot L, tokens per window LW, ws compile-time (shifts / constant divisions),
-// shift 0 or ws/2.  ORDER 0: row-major.  1: every window in quadrant order.  2: quadrant order for the windows that wrap.
+// shift 0 or ws/2.  ORDER 0: row-major.  2: quadrant order for the windows that wrap.
 template <int L, int WS, int ORDER, int LW>
 __device__ __forceinline__ RowGeom row_geom_fast(const WinGeom& gm, int tile, int r) {
+  static_assert(ORDER == 0 || ORDER == 2, "ORDER 0 (unshifted) or 2 (shifted)");
   constexpr int N = WS * WS, G = 128 / L, RA = (WS + 1) / 2, RB = WS - RA;
   RowGeom o;
   o.g = r / L;
@@ -231,7 +236,7 @@ __device__ __forceinline__ RowGeom row_geom_fast(const WinGeom& gm, int tile, in
   }
   o.gw = b * gm.nW + wh * gm.nWw + ww;        // the window's index in the natural (un-permuted) order
   int t;
-  if (ORDER == 0 || (ORDER == 2 && !o.wraps)) {
+  if (ORDER == 0 || !o.wraps) {
     t = rem / N;
     const int pos = rem % N;
     o.rr = pos / WS;
@@ -354,6 +359,93 @@ __device__ __forceinline__ void warp_store_rows(uint8_t* stage, const uint4 (&va
 
 __device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
+}
+
+// ---------------------------------------------------------------- host side of both directions
+
+// Checks the geometry and fills *gm.  qk_scale > 0 replaces head_dim^-0.5; mask: optional dense additive mask
+// [mask_windows, N, N], or null.
+int fill_geom(WinGeom* gm, int B, int T, int H, int W, int C, int nH, int ws, int shift, float qk_scale,
+              const float* mask, int mask_windows);
+// tensor maps over a [B*T, H, W, channels] bf16 tensor: whole-window box and the four rectangle boxes
+int make_window_tmaps(WinMaps* maps, const void* base, const WinGeom& gm, int channels);
+
+// Every kernel instantiation of the forward and of the backward, X(L, WS, ORDER, GEN, LWT) (the template parameters
+// of winattn_fwd_kernel); the backward instantiates each one for SHT = 1 and 2 heads per 64-channel group.
+#define STSWIN_WINATTN_VARIANTS(X)                                                                  \
+  X(128, 7, 0, false, 98) X(128, 7, 2, false, 98) X(64, 7, 0, false, 49) X(64, 7, 2, false, 49)   \
+  X(64, 5, 0, false, 50) X(64, 5, 2, false, 50) X(32, 5, 0, false, 25) X(32, 5, 2, false, 25)     \
+  X(32, 0, 0, true, 32) X(128, 0, 0, true, 128)                                                   \
+  X(128, 8, 0, false, 128) X(128, 8, 2, false, 128) X(64, 8, 0, false, 64) X(64, 8, 2, false, 64) \
+  X(32, 4, 0, false, 32) X(32, 4, 2, false, 32)                                                   \
+  X(16, 0, 0, false, 16) X(32, 0, 0, false, 32) X(64, 0, 0, false, 64) X(128, 0, 0, false, 128)
+
+struct WinVariant {
+  int L, WS, ORDER;
+  bool GEN;
+  int LWT;
+};
+
+// The instantiation that runs a geometry.  Every variant computes the same result; the choice decides only speed.
+// backward: sets the backward kernel's gm.general and gm.perm first.
+inline WinVariant select_variant(WinGeom& gm, bool backward) {
+  if (backward) {
+    if (gm.shift > 0 && gm.ra != gm.rb) gm.general = 1;   // unequal rectangles: no static column -> position fold
+    gm.perm = gm.shift > 0 && gm.nWh > 1 && gm.nWw > 1;   // interior windows first: one token-order switch per CTA
+  }
+  const int ws = gm.ws, L = gm.L;
+  // token order of a shifted block: quadrant order only for the windows that wrap (one box per interior window
+  // measured faster than four quadrant boxes for every window, at every L)
+  const int order = gm.shift == 0 ? 0 : 2;
+  // compile-time column maps need shift 0 or ws/2 (rectangles of ceil(ws/2) and ws/2) and no dense mask
+  const bool maps = gm.mask == nullptr && (gm.shift == 0 || gm.shift == ws / 2);
+  // odd windows in padded slots (7x7 and 5x5 with one or two frames: 49 of 64 / 98 of 128 / 25 of 32 / 50 of 64 rows)
+  if (maps && ((ws == 7 && (L == 49 || L == 98)) || (ws == 5 && (L == 25 || L == 50))))
+    return {gm.slot, ws, order, false, L};
+  // look-up table with window tags: the warp's 32-column band for windows of 4 / 8 tokens, else the whole row
+  if (gm.general) return gm.slot <= 8 && 32 % gm.slot == 0 ? WinVariant{32, 0, 0, true, 32} : WinVariant{128, 0, 0, true, 128};
+  // the shipped geometries: ws 8 or 4, one or two frames per window
+  if (maps && ((ws == 8 && (L == 128 || L == 64)) || (ws == 4 && L == 32))) return {L, ws, order, false, L};
+  return {L, 0, 0, false, L};   // look-up table per column
+}
+
+template <int L_, int WS_, int ORDER_, bool GEN_, int LWT_>
+struct WinKernel {
+  static constexpr int L = L_, WS = WS_, ORDER = ORDER_, LWT = LWT_;
+  static constexpr bool GEN = GEN_;
+};
+
+// launch(WinKernel<v's template parameters>{}) for a listed variant v
+template <typename F>
+int dispatch_variant(const WinVariant& v, F&& launch) {
+#define STSWIN_DISPATCH(L_, WS_, ORDER_, GEN_, LWT_)                                          \
+  if (v.L == L_ && v.WS == WS_ && v.ORDER == ORDER_ && v.GEN == GEN_ && v.LWT == LWT_) \
+    return launch(WinKernel<L_, WS_, ORDER_, GEN_, LWT_>{});
+  STSWIN_WINATTN_VARIANTS(STSWIN_DISPATCH)
+#undef STSWIN_DISPATCH
+  return set_error(kErrUnsupported, "winattn: no kernel instantiation L=%d WS=%d ORDER=%d GEN=%d LWT=%d", v.L, v.WS,
+                   v.ORDER, int(v.GEN), v.LWT);
+}
+
+// CTAs of a launch: at most one per SM, and a multiple of the head groups (every CTA keeps one head group: its bias
+// tables live in shared memory).  The work items are a multiple of the head groups, so the grid holds at least one
+// of each unless there are more head groups than SMs.
+inline int winattn_grid(const WinGeom& gm, int* grid) {
+  const int items = gm.num_tiles * gm.ngrp;
+  *grid = items < num_sms() ? items : num_sms();
+  *grid -= *grid % gm.ngrp;
+  if (*grid < gm.ngrp) return set_error(kErrUnsupported, "winattn: %d head groups exceed the SM count", gm.ngrp);
+  return kOk;
+}
+
+template <typename... KArgs, typename... Args>
+int launch_winattn(void (*kern)(KArgs...), const WinGeom& gm, int threads, int smem, cudaStream_t stream, Args... args) {
+  int grid, rc;
+  if ((rc = winattn_grid(gm, &grid)) != kOk) return rc;
+  STSWIN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  STSWIN_CUDA(launch_pdl(kern, dim3(grid), dim3(threads), (size_t)smem, stream, args...));
+  STSWIN_CUDA(cudaGetLastError());
+  return kOk;
 }
 
 }  // namespace stswin

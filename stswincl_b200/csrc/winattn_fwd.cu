@@ -17,7 +17,6 @@
 // both; a softmax and an epilogue warp share each SM sub-partition, so the MUFU-heavy softmax of
 // item k overlaps the TMEM / store-heavy drain of item k-1).  Operand chunks stream through a ring
 // of 16 KB slots.  The tensor core runs one item ahead: S(k+1) is issued before P V(k).
-#include <cstdlib>
 #include <type_traits>
 
 #include "winattn_common.cuh"
@@ -30,13 +29,10 @@ namespace {
 constexpr int NQK = 6;                         // ring of Q / K chunks (consumed by S = Q K^T)
 constexpr int NV = 4;                          // ring of V chunks (consumed by O = P V)
 constexpr int NSLOT = NQK + NV;
-constexpr int SLOT_BYTES = 128 * 128;          // 128 rows x 64 bf16
 constexpr int P_BYTES = 2 * SLOT_BYTES;        // P [128 x 128] bf16 as two K-major halves
 constexpr int STG_BYTES = 4 * 4096;             // per-warp output transposition areas (epilogue warps)
-constexpr int TAB_MAX = 15 * 15;               // (2*ws-1)^2 for ws <= 8
 constexpr int NUM_THREADS = 384;               // warpgroup 0: producer, MMA issuer (+2 idle); 1: softmax; 2: epilogue
 constexpr int SMEM_BYTES = 1024 + NSLOT * SLOT_BYTES + P_BYTES + STG_BYTES + 128 * 4 + 2 * (TAB_MAX + 1) * 4 + 512 * 4 + 256;
-constexpr float kMaskLog2e = -100.0f * 1.4426950408889634f;
 STSWIN_TRACE_DECL(g_trace_fwd)
 
 // L   : window columns a thread walks (16/32/64/128).  GEN: the tile holds G windows of gm.L tokens with gm.L not
@@ -44,11 +40,12 @@ STSWIN_TRACE_DECL(g_trace_fwd)
 //       windows have 4 / 8 tokens and never straddle a warp, the 32-column band of its warp (L = 32) -- and keeps only
 //       the columns tagged with its own window.
 //
-// WS > 0 selects the fast softmax (compile-time geometry: slot L, LWT = T*WS*WS <= L tokens per window, whole launch
-// in one token order, or one order per window: see ORDER below).  The
+// WS > 0 selects the fast softmax (compile-time geometry: slot L, LWT = T*WS*WS <= L tokens per window; ORDER 0
+// unshifted, 2 shifted: quadrant order for the windows that wrap, row-major for the others).  The
 // column -> (relative-position key, quadrant) map is then a compile-time function of the column,
 // so the bias is one LDS at an immediate offset and the shift mask is one additive constant per
 // quadrant.  WS == 0 is the generic path (look-up table per column: dense mask, L = 16, GEN).
+// STSWIN_WINATTN_VARIANTS lists the instantiations and select_variant picks one (winattn_common.cuh).
 template <int L, int WS, int ORDER, bool GEN, int LWT>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 winattn_fwd_kernel(const __grid_constant__ WinMaps tm_qkv, __nv_bfloat16* __restrict__ out,
@@ -82,8 +79,6 @@ winattn_fwd_kernel(const __grid_constant__ WinMaps tm_qkv, __nv_bfloat16* __rest
   const int hg = blockIdx.x % gm.ngrp;              // constant per CTA: gridDim.x % ngrp == 0
   const int n_local = (num_items - int(blockIdx.x) + int(gridDim.x) - 1) / int(gridDim.x);   // items of this CTA
   const int n_units = n_local * SH;                 // unit = (item, head of the group)
-  // S of unit u+1 is issued before P V of unit u (the softmax of u+1 then never waits for a tensor-core round trip).
-  const bool lag = gm.lag != 0;
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tm_qkv.full);
@@ -225,17 +220,11 @@ winattn_fwd_kernel(const __grid_constant__ WinMaps tm_qkv, __nv_bfloat16* __rest
       }
       __syncwarp();
     };
-    if (lag) {
-      if (n_units > 0) issue_S(0);
-      for (int u = 0; u < n_units; ++u) {
-        if (u + 1 < n_units) issue_S(u + 1);
-        issue_PV(u);
-      }
-    } else {
-      for (int u = 0; u < n_units; ++u) {
-        issue_S(u);
-        issue_PV(u);
-      }
+    // S of unit u+1 is issued before P V of unit u (the softmax of u+1 then never waits for a tensor-core round trip).
+    if (n_units > 0) issue_S(0);
+    for (int u = 0; u < n_units; ++u) {
+      if (u + 1 < n_units) issue_S(u + 1);
+      issue_PV(u);
     }
    }
   } else if (warp < 8) {
@@ -340,8 +329,8 @@ winattn_fwd_kernel(const __grid_constant__ WinMaps tm_qkv, __nv_bfloat16* __rest
           }
         };
         // a warp never straddles two windows for L >= 32, so the branch is warp-uniform
-        if (ORDER == 0 || (ORDER == 2 && !rg.wraps)) softmax_fast(std::false_type{});
-        else                                         softmax_fast(std::true_type{});
+        if (ORDER == 0 || !rg.wraps) softmax_fast(std::false_type{});
+        else                         softmax_fast(std::true_type{});
       } else {
         // ---- generic path: per-column look-up table (any order, dense mask, window tags)
         named_bar_sync(1, 128);                  // everybody is done with the previous LUT
@@ -471,7 +460,8 @@ winattn_fwd_kernel(const __grid_constant__ WinMaps tm_qkv, __nv_bfloat16* __rest
 
 }  // namespace
 
-int fill_geom(WinGeom* gm, int B, int T, int H, int W, int C, int nH, int ws, int shift) {
+int fill_geom(WinGeom* gm, int B, int T, int H, int W, int C, int nH, int ws, int shift, float qk_scale,
+              const float* mask, int mask_windows) {
   STSWIN_CHECK_ARG(B > 0 && T > 0 && H > 0 && W > 0 && C > 0 && nH > 0 && ws > 0, "winattn: non-positive dimension");
   STSWIN_CHECK_ARG(H % ws == 0 && W % ws == 0, "winattn: H=%d, W=%d must be multiples of the window size %d", H, W, ws);
   STSWIN_CHECK_ARG(C % nH == 0, "winattn: C=%d not divisible by num_heads=%d", C, nH);
@@ -498,8 +488,8 @@ int fill_geom(WinGeom* gm, int B, int T, int H, int W, int C, int nH, int ws, in
   gm->ngrp = nH / gm->SH;
   gm->gch = gm->SH * gm->hd;
   gm->nc = gm->gch / 64;
-  gm->scale_log2e = 1.4426950408889634f / sqrtf((float)gm->hd);
-  gm->scale = 1.0f / sqrtf((float)gm->hd);
+  gm->scale_log2e = qk_scale > 0.f ? qk_scale * 1.4426950408889634f : 1.4426950408889634f / sqrtf((float)gm->hd);
+  gm->scale = qk_scale > 0.f ? qk_scale : 1.0f / sqrtf((float)gm->hd);
   gm->ra = ws - shift; gm->rb = shift;
   {
     int off = 0;
@@ -511,13 +501,13 @@ int fill_geom(WinGeom* gm, int B, int T, int H, int W, int C, int nH, int ws, in
   }
   gm->uniform_quad = 0;
   gm->perm = 0;
-  gm->lag = 1;
-  gm->mask = nullptr; gm->mask_nw = 0;
+  gm->mask = mask; gm->mask_nw = mask_windows;
   // exact multiply-shift division of window indices (row_geom_fast)
   if ((unsigned long long)gm->total_windows * (unsigned long long)gm->nW >= (1ull << 32))
     return set_error(kErrUnsupported, "winattn: %d windows exceed the supported index range", gm->total_windows);
   gm->mg_nW = ((1ull << 32) + gm->nW - 1) / gm->nW;
   gm->mg_nWw = ((1ull << 32) + gm->nWw - 1) / gm->nWw;
+  STSWIN_CHECK_ARG(mask == nullptr || mask_windows > 0, "winattn: mask given with mask_windows <= 0");
   return kOk;
 }
 
@@ -538,15 +528,9 @@ int make_window_tmaps(WinMaps* maps, const void* base, const WinGeom& gm, int ch
   return kOk;
 }
 
-template <typename K>
-static int set_smem(K kern, int bytes) {
-  STSWIN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
-  return kOk;
-}
-
 long winattn_lse_elems(int B, int T, int H, int W, int C, int nH, int ws) {
   WinGeom gm;
-  if (fill_geom(&gm, B, T, H, W, C, nH, ws, 0) != kOk) return -1;
+  if (fill_geom(&gm, B, T, H, W, C, nH, ws, 0, 0.f, nullptr, 0) != kOk) return -1;
   return (long)gm.num_tiles * gm.nH * 128;
 }
 
@@ -561,60 +545,16 @@ int winattn_fwd(const void* qkv, const float* bias_table, void* out, float* lse2
                 int nH, int ws, int shift, float qk_scale, const float* mask, int mask_windows, cudaStream_t stream) {
   STSWIN_CHECK_ARG(qkv && bias_table && out && lse2, "winattn_fwd: null pointer");
   WinGeom gm;
-  int rc = fill_geom(&gm, B, T, H, W, C, nH, ws, shift);
+  int rc = fill_geom(&gm, B, T, H, W, C, nH, ws, shift, qk_scale, mask, mask_windows);
   if (rc != kOk) return rc;
-  if (qk_scale > 0.f) { gm.scale = qk_scale; gm.scale_log2e = qk_scale * 1.4426950408889634f; }
-  STSWIN_CHECK_ARG(mask == nullptr || mask_windows > 0, "winattn: mask given with mask_windows <= 0");
-  gm.mask = mask; gm.mask_nw = mask_windows;
-  if (const char* e = getenv("STSWIN_FWD_LAG")) gm.lag = atoi(e);      // A/B switch (tools/sweep_attn.py)
   STSWIN_CHECK_ARG((reinterpret_cast<uintptr_t>(out) & 15) == 0, "winattn_fwd: out must be 16-byte aligned");
   WinMaps tq;
   if ((rc = make_window_tmaps(&tq, qkv, gm, 3 * C)) != kOk) return rc;
-  const int items = gm.num_tiles * gm.ngrp;
-  int grid = items < num_sms() ? items : num_sms();
-  grid -= grid % gm.ngrp;                 // every CTA keeps one head group (its bias tables live in smem)
-#define STSWIN_LAUNCH_FWD_P(LL, WW, QQ, GG, PP)                                                                \
-  {                                                                                                            \
-    if ((rc = set_smem(winattn_fwd_kernel<LL, WW, QQ, GG, PP>, SMEM_BYTES)) != kOk) return rc;                 \
-    STSWIN_CUDA(launch_pdl(winattn_fwd_kernel<LL, WW, QQ, GG, PP>, dim3(grid), dim3(NUM_THREADS), (size_t)SMEM_BYTES, stream, tq,  \
-                           static_cast<__nv_bfloat16*>(out), bias_table, lse2, gm));                             \
-  }
-#define STSWIN_LAUNCH_FWD(LL, WW, QQ, GG) STSWIN_LAUNCH_FWD_P(LL, WW, QQ, GG, LL)
-  // fast softmax: the shipped geometries (ws 8 or 4, 1 or 2 frames per window, shift 0 or ws/2, no dense mask)
-  const bool fast = !gm.general && mask == nullptr && (shift == 0 || 2 * shift == ws) &&
-                    ((ws == 8 && (gm.L == 128 || gm.L == 64)) || (ws == 4 && gm.L == 32));
-  // token order of a shifted block: quadrant order only for the windows that wrap (one box per
-  // interior window measured faster than four quadrant boxes for every window, at every L)
-  const int order = shift == 0 ? 0 : (gm.uniform_quad ? 1 : 2);
-  // odd windows in padded slots (7x7 and 5x5 with one or two frames: 49 of 64 / 98 of 128 / 25 of 32 / 50 of 64 rows),
-  // shift 0 or ws/2: compile-time maps as well
-  const bool fastp = gm.general && mask == nullptr && (shift == 0 || shift == ws / 2) && order != 1 &&
-                     ((ws == 7 && (gm.L == 49 || gm.L == 98)) || (ws == 5 && (gm.L == 25 || gm.L == 50)));
-  if (fastp && ws == 7 && gm.L == 98 && order == 0) STSWIN_LAUNCH_FWD_P(128, 7, 0, false, 98)
-  else if (fastp && ws == 7 && gm.L == 98) STSWIN_LAUNCH_FWD_P(128, 7, 2, false, 98)
-  else if (fastp && ws == 7 && order == 0) STSWIN_LAUNCH_FWD_P(64, 7, 0, false, 49)
-  else if (fastp && ws == 7) STSWIN_LAUNCH_FWD_P(64, 7, 2, false, 49)
-  else if (fastp && gm.L == 50 && order == 0) STSWIN_LAUNCH_FWD_P(64, 5, 0, false, 50)
-  else if (fastp && gm.L == 50) STSWIN_LAUNCH_FWD_P(64, 5, 2, false, 50)
-  else if (fastp && order == 0) STSWIN_LAUNCH_FWD_P(32, 5, 0, false, 25)
-  else if (fastp) STSWIN_LAUNCH_FWD_P(32, 5, 2, false, 25)
-  else if (gm.general && gm.slot <= 8 && 32 % gm.slot == 0) STSWIN_LAUNCH_FWD(32, 0, 0, true)   // windows of 4 / 8 tokens
-  else if (gm.general) STSWIN_LAUNCH_FWD(128, 0, 0, true)
-  else if (fast && gm.L == 128 && order == 0) STSWIN_LAUNCH_FWD(128, 8, 0, false)
-  else if (fast && gm.L == 128 && order == 1) STSWIN_LAUNCH_FWD(128, 8, 1, false)
-  else if (fast && gm.L == 128) STSWIN_LAUNCH_FWD(128, 8, 2, false)
-  else if (fast && gm.L == 64 && order == 0) STSWIN_LAUNCH_FWD(64, 8, 0, false)
-  else if (fast && gm.L == 64) STSWIN_LAUNCH_FWD(64, 8, 2, false)
-  else if (fast && gm.L == 32 && order == 0) STSWIN_LAUNCH_FWD(32, 4, 0, false)
-  else if (fast && gm.L == 32) STSWIN_LAUNCH_FWD(32, 4, 2, false)
-  else if (gm.L == 16) STSWIN_LAUNCH_FWD(16, 0, 0, false)
-  else if (gm.L == 32) STSWIN_LAUNCH_FWD(32, 0, 0, false)
-  else if (gm.L == 64) STSWIN_LAUNCH_FWD(64, 0, 0, false)
-  else STSWIN_LAUNCH_FWD(128, 0, 0, false)
-#undef STSWIN_LAUNCH_FWD_P
-#undef STSWIN_LAUNCH_FWD
-  STSWIN_CUDA(cudaGetLastError());
-  return kOk;
+  return dispatch_variant(select_variant(gm, false), [&](auto v) {
+    using V = decltype(v);
+    return launch_winattn(winattn_fwd_kernel<V::L, V::WS, V::ORDER, V::GEN, V::LWT>, gm, NUM_THREADS, SMEM_BYTES, stream,
+                          tq, static_cast<__nv_bfloat16*>(out), bias_table, lse2, gm);
+  });
 }
 
 }  // namespace stswin
