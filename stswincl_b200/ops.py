@@ -183,6 +183,13 @@ def gemm(a: torch.Tensor, b: torch.Tensor, *, a_mn_major: bool = False, b_mn_maj
     return out
 
 
+def _wgrad_splits(n_out: int, k_in: int, tokens: int) -> int:
+    """Split-K factor of a weight-gradient GEMM dW [n_out, k_in] reduced over ``tokens`` rows: about two work items per
+    CTA pair of the 148 SMs, and at least 64 rows per split."""
+    tiles = ((n_out + 127) // 128) * ((k_in + 255) // 256)
+    return max(1, min((tokens + 63) // 64, round(2 * 148 / tiles)))
+
+
 def _mask_windows(mask: Optional[torch.Tensor], ws: int) -> int:
     if mask is None:
         return 0
@@ -245,6 +252,16 @@ def winattn_bwd(qkv: torch.Tensor, bias_table: torch.Tensor, lse2: torch.Tensor,
     return d_qkv
 
 
+def _layernorm_rows(x: torch.Tensor, patch_merge_hw):
+    """Row geometry of a LayerNorm over x: ``(M, row_len, pm, H, W, C)`` as the C ABI takes it.  Rows are the last dim of
+    x, or with ``patch_merge_hw=(H, W)`` the 2x2-gathered 4C vectors of PatchMerging (x [BT, H*W, C])."""
+    if patch_merge_hw is None:
+        return x.numel() // x.shape[-1], x.shape[-1], 0, 0, 0, 0
+    H, W = patch_merge_hw
+    C = x.shape[-1]
+    return x.numel() // C // 4, 4 * C, 1, H, W, C
+
+
 def layernorm_fwd(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps: float = 1e-5, *,
                   patch_merge_hw=None):
     """LayerNorm over the last dim of x [M, C] (bf16) -> (y bf16, mean fp32 [M], rstd fp32 [M]).
@@ -253,13 +270,7 @@ def layernorm_fwd(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps:
     gamma, beta = _al16(gamma), _al16(beta)
     _req(x, torch.bfloat16, "x"); _req(gamma, torch.float32, "gamma"); _req(beta, torch.float32, "beta")
     assert x.is_contiguous()
-    if patch_merge_hw is None:
-        M, row_len = x.numel() // x.shape[-1], x.shape[-1]
-        pm, H, W, C = 0, 0, 0, 0
-    else:
-        H, W = patch_merge_hw
-        C = x.shape[-1]
-        M, row_len, pm = x.numel() // C // 4, 4 * C, 1
+    M, row_len, pm, H, W, C = _layernorm_rows(x, patch_merge_hw)
     assert gamma.numel() == row_len and beta.numel() == row_len
     y = torch.empty((M, row_len), dtype=torch.bfloat16, device=x.device)
     mean = torch.empty(M, dtype=torch.float32, device=x.device)
@@ -278,13 +289,7 @@ def layernorm_bwd(dy: torch.Tensor, x: torch.Tensor, mean: torch.Tensor, rstd: t
     gamma = _al16(gamma)
     _req(dy, torch.bfloat16, "dy"); _req(x, torch.bfloat16, "x")
     assert dy.is_contiguous() and x.is_contiguous()
-    if patch_merge_hw is None:
-        M, row_len = x.numel() // x.shape[-1], x.shape[-1]
-        pm, H, W, C = 0, 0, 0, 0
-    else:
-        H, W = patch_merge_hw
-        C = x.shape[-1]
-        M, row_len, pm = x.numel() // C // 4, 4 * C, 1
+    M, row_len, pm, H, W, C = _layernorm_rows(x, patch_merge_hw)
     assert dy.numel() == M * row_len
     dx = torch.empty_like(x)
     if dres is not None:

@@ -80,10 +80,8 @@ def linear_wgrad(dy: torch.Tensor, x: torch.Tensor, gelu_input: bool = False) ->
     """dW [N, K] = dy^T f(x), reduced over the rows (tokens) on the tensor cores, split-K."""
     N, K, tokens = dy.shape[1], x.shape[1], dy.shape[0]
     dw = torch.zeros((N, K), dtype=_F32, device=dy.device)
-    tiles = ((N + 127) // 128) * ((K + 255) // 256)
-    splits = max(1, min((3 * tokens + 63) // 64, round(2 * 148 / tiles)))
     ops.gemm(split(dy, ROWS, SPLIT_A), split(x, ROWS, SPLIT_B, gelu=gelu_input), a_mn_major=True, b_mn_major=True,
-             mode=ops.EPI_F32_REDUCE, out=dw, k_splits=splits)
+             mode=ops.EPI_F32_REDUCE, out=dw, k_splits=ops._wgrad_splits(N, K, 3 * tokens))   # the split rows are 3x
     return dw
 
 
@@ -91,13 +89,7 @@ def layernorm_fwd(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps:
     gamma, beta = gamma.contiguous(), beta.contiguous()
     _req(x, _F32, "x")
     assert x.is_contiguous()
-    if patch_merge_hw is None:
-        M, row_len = x.numel() // x.shape[-1], x.shape[-1]
-        pm, H, W, C = 0, 0, 0, 0
-    else:
-        H, W = patch_merge_hw
-        C = x.shape[-1]
-        M, row_len, pm = x.numel() // C // 4, 4 * C, 1
+    M, row_len, pm, H, W, C = ops._layernorm_rows(x, patch_merge_hw)
     y = torch.empty((M, row_len), dtype=_F32, device=x.device)
     mean = torch.empty(M, dtype=_F32, device=x.device)
     rstd = torch.empty(M, dtype=_F32, device=x.device)
@@ -111,13 +103,7 @@ def layernorm_fwd(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps:
 def layernorm_bwd(dy, x, mean, rstd, gamma, dgamma, dbeta, dres=None, patch_merge_hw=None):
     _req(dy, _F32, "dy"); _req(x, _F32, "x")
     assert dy.is_contiguous() and x.is_contiguous()
-    if patch_merge_hw is None:
-        M, row_len = x.numel() // x.shape[-1], x.shape[-1]
-        pm, H, W, C = 0, 0, 0, 0
-    else:
-        H, W = patch_merge_hw
-        C = x.shape[-1]
-        M, row_len, pm = x.numel() // C // 4, 4 * C, 1
+    M, row_len, pm, H, W, C = ops._layernorm_rows(x, patch_merge_hw)
     dx = torch.empty_like(x)
     with _launch("f32_layernorm_bwd", 20.0 * M * row_len, x):
         st = _lib.load().stswin_f32_layernorm_bwd(dy.data_ptr(), x.data_ptr(), mean.data_ptr(), rstd.data_ptr(), gamma.data_ptr(),

@@ -21,13 +21,13 @@ per call.  There is no CPU path and no PyTorch fallback: CPU tensors raise.
 from __future__ import annotations
 
 import math
-from typing import Optional
 
 import torch
 import torch.nn as nn
 
-from . import ops
+from . import ops, ops32
 from ._lib import StswinError
+from .ops import _wgrad_splits
 from .optim import bf16_weight as _w16
 
 _BF16 = torch.bfloat16
@@ -61,18 +61,12 @@ def _shift_attn_mask(H: int, W: int, ws: int, shift: int) -> torch.Tensor:
     return torch.where(differ, torch.tensor(-100.0), torch.tensor(0.0))
 
 
-def _wgrad_splits(n_out: int, k_in: int, tokens: int) -> int:
-    tiles = ((n_out + 127) // 128) * ((k_in + 255) // 256)
-    return max(1, min((tokens + 63) // 64, round(2 * 148 / tiles)))
-
-
-def _linear_wgrad(dy2d: torch.Tensor, x2d: torch.Tensor, shape, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """dW[N_out, K_in] = dy^T x, reduced over tokens on the tensor cores (fp32, split-K).
+def _linear_wgrad(dy2d: torch.Tensor, x2d: torch.Tensor, out: torch.Tensor) -> torch.Tensor:
+    """out[N_out, K_in] = dy^T x, reduced over tokens on the tensor cores (fp32, split-K).
     ``out`` must be zero-filled (the split-K epilogue accumulates)."""
-    dw = out if out is not None else torch.zeros(shape, dtype=torch.float32, device=dy2d.device)
-    ops.gemm(dy2d, x2d, a_mn_major=True, b_mn_major=True, mode=ops.EPI_F32_REDUCE, out=dw,
-             k_splits=_wgrad_splits(shape[0], shape[1], dy2d.shape[0]))
-    return dw
+    ops.gemm(dy2d, x2d, a_mn_major=True, b_mn_major=True, mode=ops.EPI_F32_REDUCE, out=out,
+             k_splits=_wgrad_splits(out.shape[0], out.shape[1], dy2d.shape[0]))
+    return out
 
 
 def _zeros_like_many(shapes, device):
@@ -86,6 +80,66 @@ def _zeros_like_many(shapes, device):
     return [flat[o:o + n].view(s) for o, n, s in zip(offs, sizes, shapes)]
 
 
+# ---------------------------------------------------------------------------------------------------------------
+# The block's two halves on bf16 token rows x2 [rows, C], written once for the stand-alone Functions and the block.
+# ``res`` / ``dres``: a residual (rows like the output) added in the epilogue of the half's last GEMM.  Gradient
+# buffers are zero-filled fp32 (the kernels accumulate); the gradient of the half's last bias is the caller's.
+# ---------------------------------------------------------------------------------------------------------------
+def _attn_fwd(x2, shp, table, wq, b_qkv, wp, b_proj, geom, mask=None, res=None):
+    """qkv GEMM -> window attention core -> proj GEMM (+ res); ``shp`` = (Bp, T, H*W) of the rows.
+    Returns (qkv, attn, lse2, out)."""
+    H, W, nH, ws, shift, qk_scale = geom[:6]
+    C = x2.shape[1]
+    qkv = ops.gemm(x2, wq, bias=b_qkv)
+    attn, lse2 = ops.winattn_fwd(qkv.view(*shp, 3 * C), table, H, W, nH, ws, shift, qk_scale=qk_scale, mask=mask)
+    out = ops.gemm(attn.view(-1, C), wp, bias=b_proj, aux=res, mode=ops.EPI_BIAS if res is None else ops.EPI_BIAS_RES)
+    return qkv, attn, lse2, out
+
+
+def _attn_bwd(dy, shp, x2, qkv, attn, lse2, table, wq, wp, geom, d_table, d_bqkv, d_wproj, d_wqkv, mask=None,
+              need_dx=True, dres=None):
+    """Backward of ``_attn_fwd`` from dy [rows, C]: proj dgrad -> proj wgrad -> attention core -> qkv dgrad (+ dres; only
+    with ``need_dx``) -> qkv wgrad.  ``d_bqkv`` None: no qkv bias.  Returns dx [rows, C] or None."""
+    H, W, nH, ws, shift, qk_scale = geom[:6]
+    C = x2.shape[1]
+    d_attn = ops.gemm(dy, wp, b_mn_major=True)
+    _linear_wgrad(dy, attn.view(-1, C), d_wproj)
+    d_qkv = ops.winattn_bwd(qkv.view(*shp, 3 * C), table, lse2, d_attn.view(*shp, C), H, W, nH, ws, shift,
+                            d_table, d_bqkv, qk_scale=qk_scale, mask=mask)
+    dq2 = d_qkv.view(-1, 3 * C)
+    d_x = None
+    if need_dx:
+        d_x = ops.gemm(dq2, wq, b_mn_major=True, aux=dres, mode=ops.EPI_BIAS if dres is None else ops.EPI_BIAS_RES)
+    _linear_wgrad(dq2, x2, d_wqkv)
+    return d_x
+
+
+def _mlp_fwd(x2, w1, b1, w2, b2, res=None, keep_dgelu=True):
+    """fc1 + GELU -> fc2 (+ res).  With ``keep_dgelu`` the fc1 epilogue also writes GELU'(fc1 out) for the backward, one
+    byte per element when GELU_GRAD_Q8 and the width allow (a bounded multiplier; fc1 + GELU is HBM-write bound), else
+    bf16.  Returns (h, dgelu or None, y)."""
+    dgelu = None
+    if keep_dgelu:
+        q8 = GELU_GRAD_Q8 and w1.shape[0] % 16 == 0
+        dgelu = torch.empty((x2.shape[0], w1.shape[0]), dtype=torch.uint8 if q8 else _BF16, device=x2.device)
+        h = ops.gemm(x2, w1, bias=b1, mode=ops.EPI_BIAS_GELU_Q8 if q8 else ops.EPI_BIAS_GELU, out2=dgelu)
+    else:
+        h = ops.gemm(x2, w1, bias=b1, mode=ops.EPI_BIAS_GELU_FWD)
+    y = ops.gemm(h, w2, bias=b2, aux=res, mode=ops.EPI_BIAS if res is None else ops.EPI_BIAS_RES)
+    return h, dgelu, y
+
+
+def _mlp_bwd(dy, x2, h, dgelu, w1, w2, d_b1, d_w1, d_w2):
+    """Backward of ``_mlp_fwd`` from dy [rows, C_out]: fc2 dgrad times GELU' (column sums into d_b1) -> fc2 wgrad ->
+    fc1 dgrad -> fc1 wgrad.  Returns dx [rows, C_in]."""
+    du = ops.gemm(dy, w2, b_mn_major=True, mode=ops.EPI_MUL_AUX_Q8 if dgelu.dtype == torch.uint8 else ops.EPI_MUL_AUX,
+                  aux=dgelu, colsum=d_b1)
+    _linear_wgrad(dy, h, d_w2)
+    dx = ops.gemm(du, w1, b_mn_major=True)
+    _linear_wgrad(du, x2, d_w1)
+    return dx
+
+
 class _AttentionFn(torch.autograd.Function):
     """qkv Linear -> window attention core -> proj Linear on tokens in natural order.
 
@@ -93,38 +147,25 @@ class _AttentionFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x, table, w_qkv, b_qkv, w_proj, b_proj, geom, mask=None):
-        H, W, nH, ws, shift, qk_scale = geom
-        Bp, T, L, C = x.shape
-        x2 = x.reshape(-1, C)
+        x2 = x.reshape(-1, x.shape[-1])
         wq, wp = _w16(w_qkv), _w16(w_proj)
-        qkv = ops.gemm(x2, wq, bias=b_qkv)
-        attn, lse2 = ops.winattn_fwd(qkv.view(Bp, T, L, 3 * C), table, H, W, nH, ws, shift, qk_scale=qk_scale, mask=mask)
-        out = ops.gemm(attn.view(-1, C), wp, bias=b_proj)
+        qkv, attn, lse2, out = _attn_fwd(x2, x.shape[:3], table, wq, b_qkv, wp, b_proj, geom, mask)
         ctx.save_for_backward(x2, qkv, attn, lse2, table, wq, wp)
-        ctx.geom = geom
-        ctx.mask = mask
-        ctx.has_qkv_bias = b_qkv is not None
-        return out.view(Bp, T, L, C)
+        ctx.geom, ctx.mask, ctx.has_qkv_bias = geom, mask, b_qkv is not None
+        return out.view(x.shape)
 
     @staticmethod
     def backward(ctx, d_out):
         x2, qkv, attn, lse2, table, wq, wp = ctx.saved_tensors
-        H, W, nH, ws, shift, qk_scale = ctx.geom
         C = x2.shape[1]
-        Bp_T_L = d_out.shape[:3]
         d2 = d_out.contiguous().view(-1, C)
-        d_table, d_bqkv, d_bproj, d_wproj_, d_wqkv_ = _zeros_like_many([tuple(table.shape), (3 * C,), (C,), tuple(wp.shape), tuple(wq.shape)], d2.device)
+        d_table, d_bqkv, d_bproj, d_wproj, d_wqkv = _zeros_like_many([tuple(table.shape), (3 * C,), (C,), tuple(wp.shape), tuple(wq.shape)], d2.device)
         ops.colsum(d2, d_bproj)                           # proj bias gradient: one read of d_out
         if not ctx.has_qkv_bias:
             d_bqkv = None
-        d_attn = ops.gemm(d2, wp, b_mn_major=True)
-        d_wproj = _linear_wgrad(d2, attn.view(-1, C), wp.shape, d_wproj_)
-        d_qkv = ops.winattn_bwd(qkv.view(*Bp_T_L, 3 * C), table, lse2, d_attn.view(*Bp_T_L, C), H, W, nH, ws, shift,
-                                d_table, d_bqkv, qk_scale=qk_scale, mask=ctx.mask)
-        dq2 = d_qkv.view(-1, 3 * C)
-        d_x = ops.gemm(dq2, wq, b_mn_major=True)
-        d_wqkv = _linear_wgrad(dq2, x2, wq.shape, d_wqkv_)
-        return d_x.view(*Bp_T_L, C), d_table, d_wqkv, d_bqkv, d_wproj, d_bproj, None, None
+        d_x = _attn_bwd(d2, d_out.shape[:3], x2, qkv, attn, lse2, table, wq, wp, ctx.geom, d_table, d_bqkv, d_wproj, d_wqkv,
+                        ctx.mask)
+        return d_x.view(d_out.shape), d_table, d_wqkv, d_bqkv, d_wproj, d_bproj, None, None
 
 
 class _BlockFn(torch.autograd.Function):
@@ -137,70 +178,42 @@ class _BlockFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x, table, w_qkv, b_qkv, w_proj, b_proj, g1, be1, g2, be2, w_fc1, b_fc1, w_fc2, b_fc2, geom):
-        H, W, nH, ws, shift, qk_scale, eps, infer = geom
-        geom = geom[:7]
-        Bp, T, L, C = x.shape
-        x2 = x.reshape(-1, C)
+        eps = geom[6]
+        # inference (no_grad key encoders of the pre-training model, evaluation): no gelu' output, nothing kept for a backward
+        infer = geom[7] or not any(ctx.needs_input_grad)
+        x2 = x.reshape(-1, x.shape[-1])
         wq, wp, w1, w2 = _w16(w_qkv), _w16(w_proj), _w16(w_fc1), _w16(w_fc2)
-        qkv = ops.gemm(x2, wq, bias=b_qkv)
-        attn, lse2 = ops.winattn_fwd(qkv.view(Bp, T, L, 3 * C), table, H, W, nH, ws, shift, qk_scale=qk_scale)
-        y = ops.gemm(attn.view(-1, C), wp, bias=b_proj, aux=x2, mode=ops.EPI_BIAS_RES)
+        qkv, attn, lse2, y = _attn_fwd(x2, x.shape[:3], table, wq, b_qkv, wp, b_proj, geom, res=x2)
         yn, mean2, rstd2 = ops.layernorm_fwd(y, g2, be2, eps)
-        if infer or not any(ctx.needs_input_grad):
-            # inference (no_grad key encoders of the pre-training model, evaluation): no gelu' output,
-            # nothing kept for a backward
-            h = ops.gemm(yn, w1, bias=b_fc1, mode=ops.EPI_BIAS_GELU_FWD)
-            z = ops.gemm(h, w2, bias=b_fc2, aux=y, mode=ops.EPI_BIAS_RES)
-            out, _, _ = ops.layernorm_fwd(z, g1, be1, eps)
-            return out.view(Bp, T, L, C)
-        # gelu'(fc1 out) for the backward, one byte per element (a bounded multiplier; fc1 + GELU is HBM-write bound)
-        q8 = GELU_GRAD_Q8 and w1.shape[0] % 16 == 0
-        dgelu = torch.empty((x2.shape[0], w1.shape[0]), dtype=torch.uint8 if q8 else _BF16, device=x.device)
-        h = ops.gemm(yn, w1, bias=b_fc1, mode=ops.EPI_BIAS_GELU_Q8 if q8 else ops.EPI_BIAS_GELU, out2=dgelu)
-        z = ops.gemm(h, w2, bias=b_fc2, aux=y, mode=ops.EPI_BIAS_RES)
+        h, dgelu, z = _mlp_fwd(yn, w1, b_fc1, w2, b_fc2, res=y, keep_dgelu=not infer)
         out, mean1, rstd1 = ops.layernorm_fwd(z, g1, be1, eps)
-        ctx.save_for_backward(x2, qkv, attn, lse2, y, yn, mean2, rstd2, dgelu, h, z, mean1, rstd1,
-                              table, wq, wp, w1, w2, g1, g2)
-        ctx.geom = geom
-        ctx.has_qkv_bias = b_qkv is not None
-        return out.view(Bp, T, L, C)
+        if not infer:
+            ctx.save_for_backward(x2, qkv, attn, lse2, y, yn, mean2, rstd2, dgelu, h, z, mean1, rstd1,
+                                  table, wq, wp, w1, w2, g1, g2)
+            ctx.geom, ctx.has_qkv_bias = geom[:7], b_qkv is not None
+        return out.view(x.shape)
 
     @staticmethod
     def backward(ctx, d_out):
         (x2, qkv, attn, lse2, y, yn, mean2, rstd2, dgelu, h, z, mean1, rstd1,
          table, wq, wp, w1, w2, g1, g2) = ctx.saved_tensors
-        H, W, nH, ws, shift, qk_scale, eps = ctx.geom
         C = x2.shape[1]
-        shp = d_out.shape[:3]
-        dev = x2.device
         d2 = d_out.contiguous().view(-1, C)
-        (d_g1, d_be1, d_bfc2, d_bfc1, d_g2, d_be2, d_bproj, d_table, d_bqkv, d_wfc2_, d_wfc1_, d_wproj_, d_wqkv_) = \
+        (d_g1, d_be1, d_bfc2, d_bfc1, d_g2, d_be2, d_bproj, d_table, d_bqkv, d_wfc2, d_wfc1, d_wproj, d_wqkv) = \
             _zeros_like_many([(C,), (C,), (C,), (w1.shape[0],), (C,), (C,), (C,), tuple(table.shape), (3 * C,),
-                              tuple(w2.shape), tuple(w1.shape), tuple(wp.shape), tuple(wq.shape)], dev)
+                              tuple(w2.shape), tuple(w1.shape), tuple(wp.shape), tuple(wq.shape)], d2.device)
         if not ctx.has_qkv_bias:
             d_bqkv = None
-        # out = norm1(z)
+        # out = norm1(z); z = y + mlp(yn), the fc2 bias gradient is the column sums of dz
         dz = ops.layernorm_bwd(d2, z, mean1, rstd1, g1, d_g1, d_be1, dx_colsum=d_bfc2)
-        # z = y + h W2^T + b2 ; h = gelu(u), and the forward stored gelu'(u)
-        du = ops.gemm(dz, w2, b_mn_major=True, mode=ops.EPI_MUL_AUX_Q8 if dgelu.dtype == torch.uint8 else ops.EPI_MUL_AUX,
-                      aux=dgelu, colsum=d_bfc1)
-        d_wfc2 = _linear_wgrad(dz, h, w2.shape, d_wfc2_)
-        # u = yn W1^T + b1 ; yn = norm2(y)
-        dyn = ops.gemm(du, w1, b_mn_major=True)
-        d_wfc1 = _linear_wgrad(du, yn, w1.shape, d_wfc1_)
+        dyn = _mlp_bwd(dz, yn, h, dgelu, w1, w2, d_bfc1, d_wfc1, d_wfc2)
+        # yn = norm2(y); y = x + attn(x), the proj bias gradient is the column sums of dy
         dy = ops.layernorm_bwd(dyn, y, mean2, rstd2, g2, d_g2, d_be2, dres=dz, dx_colsum=d_bproj)
-        # y = x + attn Wp^T + bp
-        d_attn = ops.gemm(dy, wp, b_mn_major=True)
-        d_wproj = _linear_wgrad(dy, attn.view(-1, C), wp.shape, d_wproj_)
-        d_qkv = ops.winattn_bwd(qkv.view(*shp, 3 * C), table, lse2, d_attn.view(*shp, C), H, W, nH, ws, shift,
-                                d_table, d_bqkv, qk_scale=qk_scale)
-        dq2 = d_qkv.view(-1, 3 * C)
-        d_x = None
-        if ctx.needs_input_grad[0]:          # the first block of a head fed with features that carry no gradient skips this GEMM
-            d_x = ops.gemm(dq2, wq, b_mn_major=True, mode=ops.EPI_BIAS_RES, aux=dy).view(*shp, C)      # + residual path
-        d_wqkv = _linear_wgrad(dq2, x2, wq.shape, d_wqkv_)
-        return (d_x, d_table, d_wqkv, d_bqkv, d_wproj, d_bproj, d_g1, d_be1, d_g2, d_be2,
-                d_wfc1, d_bfc1, d_wfc2, d_bfc2, None)
+        # the first block of a head fed with features that carry no gradient skips the qkv dgrad
+        d_x = _attn_bwd(dy, d_out.shape[:3], x2, qkv, attn, lse2, table, wq, wp, ctx.geom, d_table, d_bqkv, d_wproj, d_wqkv,
+                        need_dx=ctx.needs_input_grad[0], dres=dy)
+        return (None if d_x is None else d_x.view(d_out.shape), d_table, d_wqkv, d_bqkv, d_wproj, d_bproj,
+                d_g1, d_be1, d_g2, d_be2, d_wfc1, d_bfc1, d_wfc2, d_bfc2, None)
 
 
 class _PatchMergeFn(torch.autograd.Function):
@@ -224,7 +237,7 @@ class _PatchMergeFn(torch.autograd.Function):
         B, T, L, C = x.shape
         d2 = d_out.contiguous().view(-1, wr.shape[0])
         dxn = ops.gemm(d2, wr, b_mn_major=True)
-        d_w = _linear_wgrad(d2, xn, wr.shape)
+        d_w = _linear_wgrad(d2, xn, torch.zeros(wr.shape, dtype=torch.float32, device=d2.device))
         d_gamma = torch.zeros(4 * C, dtype=torch.float32, device=x.device)
         d_beta = torch.zeros_like(d_gamma)
         dx = ops.layernorm_bwd(dxn, x.reshape(B * T, L, C), mean, rstd, gamma, d_gamma, d_beta, patch_merge_hw=(H, W))
@@ -255,10 +268,23 @@ class _FnCtx:
         self.saved_tensors = tensors
 
 
+def _mid_frames(x: torch.Tensor, blocks) -> torch.Tensor:
+    """``cat([x[:, :1], blocks(x[:, 1:3]), x[:, 3:]])`` for x [B, 4, L, C] without a ``cat``: frames 1..2 are copied out
+    and run through ``blocks``, and the output is assembled from the result and frames 0 / 3 of x."""
+    B, _, L, C = x.shape
+    xm = torch.empty((B, 2, L, C), dtype=x.dtype, device=x.device)
+    ops.copy_frames(xm, x[:, 1:3])
+    y = blocks(xm)
+    out = torch.empty_like(x)
+    ops.copy_frames(out[:, 0], x[:, 0])
+    ops.copy_frames(out[:, 3], x[:, 3])
+    ops.copy_frames(out[:, 1:3], y)
+    return out
+
+
 class _MidLayerFn(torch.autograd.Function):
     """The middle layer of a stage (swin_512.py:302-307): ``cat([x[:, :1], blk1(blk0(x[:, 1:3])), x[:, 3:]])`` as ONE
-    autograd node.  Forward: frames 1..2 are copied out, run through the two blocks, and the output is assembled from
-    the block result and frames 0 / 3 of x (no ``cat``).  Backward: the incoming gradient is only read; the gradient of
+    autograd node; the forward is ``_mid_frames``.  Backward: the incoming gradient is only read; the gradient of
     x is a fresh buffer filled from three sources (frames 0 / 3 of d_out, the blocks' input gradient for frames 1..2),
     so there is no zero-fill and no gradient accumulation for the pass-through frames."""
 
@@ -267,17 +293,9 @@ class _MidLayerFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, geom0, geom1, *params):
         n = _MidLayerFn.N_BLOCK_ARGS
-        B, _, L, C = x.shape
-        xm = torch.empty((B, 2, L, C), dtype=x.dtype, device=x.device)
-        ops.copy_frames(xm, x[:, 1:3])
         c0, c1 = _FnCtx(n + 2), _FnCtx(n + 2)
-        blk = _BlockFn32 if x.dtype == torch.float32 else _BlockFn
-        ctx.blk = blk
-        y = blk.forward(c1, blk.forward(c0, xm, *params[:n], geom0), *params[n:], geom1)
-        out = torch.empty_like(x)
-        ops.copy_frames(out[:, 0], x[:, 0])
-        ops.copy_frames(out[:, 3], x[:, 3])
-        ops.copy_frames(out[:, 1:3], y)
+        blk = ctx.blk = _BLOCK_FNS[x.dtype]
+        out = _mid_frames(x, lambda xm: blk.forward(c1, blk.forward(c0, xm, *params[:n], geom0), *params[n:], geom1))
         ctx.blocks = (c0, c1)
         return out
 
@@ -304,10 +322,7 @@ class _MlpFn(torch.autograd.Function):
     def forward(ctx, x, w1, b1, w2, b2):
         x2 = x.reshape(-1, x.shape[-1])
         w1b, w2b = _w16(w1), _w16(w2)
-        q8 = GELU_GRAD_Q8 and w1b.shape[0] % 16 == 0
-        dgelu = torch.empty((x2.shape[0], w1b.shape[0]), dtype=torch.uint8 if q8 else _BF16, device=x.device)
-        h = ops.gemm(x2, w1b, bias=b1, mode=ops.EPI_BIAS_GELU_Q8 if q8 else ops.EPI_BIAS_GELU, out2=dgelu)
-        y = ops.gemm(h, w2b, bias=b2)
+        h, dgelu, y = _mlp_fwd(x2, w1b, b1, w2b, b2)
         ctx.save_for_backward(x2, h, dgelu, w1b, w2b)
         return y.view(*x.shape[:-1], w2b.shape[0])
 
@@ -315,13 +330,9 @@ class _MlpFn(torch.autograd.Function):
     def backward(ctx, dy):
         x2, h, dgelu, w1b, w2b = ctx.saved_tensors
         d2 = dy.contiguous().view(-1, w2b.shape[0])
-        d_b2, d_b1, d_w2_, d_w1_ = _zeros_like_many([(w2b.shape[0],), (w1b.shape[0],), tuple(w2b.shape), tuple(w1b.shape)], d2.device)
+        d_b2, d_b1, d_w2, d_w1 = _zeros_like_many([(w2b.shape[0],), (w1b.shape[0],), tuple(w2b.shape), tuple(w1b.shape)], d2.device)
         ops.colsum(d2, d_b2)
-        du = ops.gemm(d2, w2b, b_mn_major=True, mode=ops.EPI_MUL_AUX_Q8 if dgelu.dtype == torch.uint8 else ops.EPI_MUL_AUX,
-                      aux=dgelu, colsum=d_b1)
-        d_w2 = _linear_wgrad(d2, h, w2b.shape, d_w2_)
-        dx = ops.gemm(du, w1b, b_mn_major=True)
-        d_w1 = _linear_wgrad(du, x2, w1b.shape, d_w1_)
+        dx = _mlp_bwd(d2, x2, h, dgelu, w1b, w2b, d_b1, d_w1, d_w2)
         return dx.view(*dy.shape[:-1], w1b.shape[1]), d_w1, d_b1, d_w2, d_b2
 
 
@@ -354,42 +365,71 @@ def _zeros_f32(shape, dev):
     return torch.zeros(shape, dtype=torch.float32, device=dev)
 
 
+# The two halves again over ops32 (fp32 rows), written once for the stand-alone Functions and the block.  They differ
+# from the bf16 ones in what they fuse: the fc2 GEMM applies GELU to its split input (u is kept, not GELU'(u)) and the
+# bias gradients are separate column sums.
+def _attn_fwd32(x2, shp, table, w_qkv, b_qkv, w_proj, b_proj, geom, mask=None, res=None):
+    """``_attn_fwd`` in fp32.  Returns (qkv, attn, lse, out)."""
+    H, W, nH, ws, shift, qk_scale = geom[:6]
+    C = x2.shape[1]
+    qkv = ops32.linear(x2, w_qkv, b_qkv)
+    attn, lse = ops32.winattn_fwd(qkv.view(*shp, 3 * C), table, H, W, nH, ws, shift, qk_scale, mask)
+    return qkv, attn, lse, ops32.linear(attn.view(-1, C), w_proj, b_proj, res=res)
+
+
+def _attn_bwd32(dy, shp, x2, qkv, attn, lse, table, w_qkv, w_proj, geom, has_qkv_bias, mask=None, dres=None):
+    """``_attn_bwd`` in fp32, from dy [rows, C].  Returns (dx (+ dres), d_table, d_wqkv, d_bqkv or None, d_wproj, d_bproj)."""
+    H, W, nH, ws, shift, qk_scale = geom[:6]
+    C = x2.shape[1]
+    dev = dy.device
+    d_bproj = ops32.colsum(dy, _zeros_f32((C,), dev))
+    d_attn = ops32.linear_dgrad(dy, w_proj)
+    d_wproj = ops32.linear_wgrad(dy, attn.view(-1, C))
+    d_table = _zeros_f32(tuple(table.shape), dev)
+    d_qkv = ops32.winattn_bwd(qkv.view(*shp, 3 * C), table, attn, lse, d_attn.view(*shp, C), H, W, nH, ws, shift, d_table,
+                              qk_scale, mask)
+    dq2 = d_qkv.view(-1, 3 * C)
+    d_bqkv = ops32.colsum(dq2, _zeros_f32((3 * C,), dev)) if has_qkv_bias else None
+    d_x = ops32.linear_dgrad(dq2, w_qkv, res=dres)
+    d_wqkv = ops32.linear_wgrad(dq2, x2)
+    return d_x, d_table, d_wqkv, d_bqkv, d_wproj, d_bproj
+
+
+def _mlp_fwd32(x2, w1, b1, w2, b2, res=None):
+    """fc1 -> GELU -> fc2 (+ res) in fp32.  Returns (u = fc1 out, y)."""
+    u = ops32.linear(x2, w1, b1)
+    return u, ops32.linear(u, w2, b2, res=res, gelu_input=True)
+
+
+def _mlp_bwd32(dy, x2, u, w1, w2):
+    """Backward of ``_mlp_fwd32`` from dy [rows, C_out].  Returns (dx, d_w1, d_b1, d_w2, d_b2)."""
+    dev = dy.device
+    d_b2 = ops32.colsum(dy, _zeros_f32((w2.shape[0],), dev))
+    dh = ops32.linear_dgrad(dy, w2)
+    d_w2 = ops32.linear_wgrad(dy, u, gelu_input=True)
+    du = ops32.mul_gelu_grad(dh, u)
+    d_b1 = ops32.colsum(du, _zeros_f32((w1.shape[0],), dev))
+    dx = ops32.linear_dgrad(du, w1)
+    d_w1 = ops32.linear_wgrad(du, x2)
+    return dx, d_w1, d_b1, d_w2, d_b2
+
+
 class _AttentionFn32(torch.autograd.Function):
     """``_AttentionFn`` in the fp32-accurate mode: x [Bp, T, H*W, C] fp32."""
 
     @staticmethod
     def forward(ctx, x, table, w_qkv, b_qkv, w_proj, b_proj, geom, mask=None):
-        from . import ops32 as o32
-        H, W, nH, ws, shift, qk_scale = geom
-        Bp, T, L, C = x.shape
-        x2 = x.reshape(-1, C)
-        qkv = o32.linear(x2, w_qkv, b_qkv)
-        attn, lse = o32.winattn_fwd(qkv.view(Bp, T, L, 3 * C), table, H, W, nH, ws, shift, qk_scale, mask)
-        out = o32.linear(attn.view(-1, C), w_proj, b_proj)
+        x2 = x.reshape(-1, x.shape[-1])
+        qkv, attn, lse, out = _attn_fwd32(x2, x.shape[:3], table, w_qkv, b_qkv, w_proj, b_proj, geom, mask)
         ctx.save_for_backward(x2, qkv, attn, lse, table, w_qkv, w_proj)
         ctx.geom, ctx.mask, ctx.has_qkv_bias = geom, mask, b_qkv is not None
-        return out.view(Bp, T, L, C)
+        return out.view(x.shape)
 
     @staticmethod
     def backward(ctx, d_out):
-        from . import ops32 as o32
-        x2, qkv, attn, lse, table, w_qkv, w_proj = ctx.saved_tensors
-        H, W, nH, ws, shift, qk_scale = ctx.geom
-        C = x2.shape[1]
-        shp = d_out.shape[:3]
-        d2 = d_out.contiguous().view(-1, C)
-        dev = d2.device
-        d_bproj = o32.colsum(d2, _zeros_f32((C,), dev))
-        d_attn = o32.linear_dgrad(d2, w_proj)
-        d_wproj = o32.linear_wgrad(d2, attn.view(-1, C))
-        d_table = _zeros_f32(tuple(table.shape), dev)
-        d_qkv = o32.winattn_bwd(qkv.view(*shp, 3 * C), table, attn, lse, d_attn.view(*shp, C), H, W, nH, ws, shift, d_table,
-                                qk_scale, ctx.mask)
-        dq2 = d_qkv.view(-1, 3 * C)
-        d_bqkv = o32.colsum(dq2, _zeros_f32((3 * C,), dev)) if ctx.has_qkv_bias else None
-        d_x = o32.linear_dgrad(dq2, w_qkv)
-        d_wqkv = o32.linear_wgrad(dq2, x2)
-        return d_x.view(*shp, C), d_table, d_wqkv, d_bqkv, d_wproj, d_bproj, None, None
+        d2 = d_out.contiguous().view(-1, d_out.shape[-1])
+        d_x, *grads = _attn_bwd32(d2, d_out.shape[:3], *ctx.saved_tensors, ctx.geom, ctx.has_qkv_bias, ctx.mask)
+        return (d_x.view(d_out.shape), *grads, None, None)
 
 
 class _BlockFn32(torch.autograd.Function):
@@ -397,51 +437,29 @@ class _BlockFn32(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x, table, w_qkv, b_qkv, w_proj, b_proj, g1, be1, g2, be2, w_fc1, b_fc1, w_fc2, b_fc2, geom):
-        from . import ops32 as o32
-        H, W, nH, ws, shift, qk_scale, eps, infer = geom
-        Bp, T, L, C = x.shape
-        x2 = x.reshape(-1, C)
-        qkv = o32.linear(x2, w_qkv, b_qkv)
-        attn, lse = o32.winattn_fwd(qkv.view(Bp, T, L, 3 * C), table, H, W, nH, ws, shift, qk_scale)
-        y = o32.linear(attn.view(-1, C), w_proj, b_proj, res=x2)
-        yn, mean2, rstd2 = o32.layernorm_fwd(y, g2, be2, eps)
-        u = o32.linear(yn, w_fc1, b_fc1)
-        z = o32.linear(u, w_fc2, b_fc2, res=y, gelu_input=True)
-        out, mean1, rstd1 = o32.layernorm_fwd(z, g1, be1, eps)
+        eps, infer = geom[6], geom[7]
+        x2 = x.reshape(-1, x.shape[-1])
+        qkv, attn, lse, y = _attn_fwd32(x2, x.shape[:3], table, w_qkv, b_qkv, w_proj, b_proj, geom, res=x2)
+        yn, mean2, rstd2 = ops32.layernorm_fwd(y, g2, be2, eps)
+        u, z = _mlp_fwd32(yn, w_fc1, b_fc1, w_fc2, b_fc2, res=y)
+        out, mean1, rstd1 = ops32.layernorm_fwd(z, g1, be1, eps)
         if not infer:
             ctx.save_for_backward(x2, qkv, attn, lse, y, yn, mean2, rstd2, u, z, mean1, rstd1, table, w_qkv, w_proj, w_fc1, w_fc2, g1, g2)
             ctx.geom, ctx.has_qkv_bias = geom[:7], b_qkv is not None
-        return out.view(Bp, T, L, C)
+        return out.view(x.shape)
 
     @staticmethod
     def backward(ctx, d_out):
-        from . import ops32 as o32
         (x2, qkv, attn, lse, y, yn, mean2, rstd2, u, z, mean1, rstd1, table, w_qkv, w_proj, w_fc1, w_fc2, g1, g2) = ctx.saved_tensors
-        H, W, nH, ws, shift, qk_scale, eps = ctx.geom
         C = x2.shape[1]
-        shp = d_out.shape[:3]
-        dev = x2.device
         d2 = d_out.contiguous().view(-1, C)
-        d_g1, d_be1, d_g2, d_be2 = (_zeros_f32((C,), dev) for _ in range(4))
-        dz = o32.layernorm_bwd(d2, z, mean1, rstd1, g1, d_g1, d_be1)
-        d_bfc2 = o32.colsum(dz, _zeros_f32((C,), dev))
-        dh = o32.linear_dgrad(dz, w_fc2)
-        d_wfc2 = o32.linear_wgrad(dz, u, gelu_input=True)
-        du = o32.mul_gelu_grad(dh, u)
-        d_bfc1 = o32.colsum(du, _zeros_f32((w_fc1.shape[0],), dev))
-        dyn = o32.linear_dgrad(du, w_fc1)
-        d_wfc1 = o32.linear_wgrad(du, yn)
-        dy = o32.layernorm_bwd(dyn, y, mean2, rstd2, g2, d_g2, d_be2, dres=dz)
-        d_bproj = o32.colsum(dy, _zeros_f32((C,), dev))
-        d_attn = o32.linear_dgrad(dy, w_proj)
-        d_wproj = o32.linear_wgrad(dy, attn.view(-1, C))
-        d_table = _zeros_f32(tuple(table.shape), dev)
-        d_qkv = o32.winattn_bwd(qkv.view(*shp, 3 * C), table, attn, lse, d_attn.view(*shp, C), H, W, nH, ws, shift, d_table, qk_scale)
-        dq2 = d_qkv.view(-1, 3 * C)
-        d_bqkv = o32.colsum(dq2, _zeros_f32((3 * C,), dev)) if ctx.has_qkv_bias else None
-        d_x = o32.linear_dgrad(dq2, w_qkv, res=dy)
-        d_wqkv = o32.linear_wgrad(dq2, x2)
-        return (d_x.view(*shp, C), d_table, d_wqkv, d_bqkv, d_wproj, d_bproj, d_g1, d_be1, d_g2, d_be2,
+        d_g1, d_be1, d_g2, d_be2 = (_zeros_f32((C,), d2.device) for _ in range(4))
+        dz = ops32.layernorm_bwd(d2, z, mean1, rstd1, g1, d_g1, d_be1)
+        dyn, d_wfc1, d_bfc1, d_wfc2, d_bfc2 = _mlp_bwd32(dz, yn, u, w_fc1, w_fc2)
+        dy = ops32.layernorm_bwd(dyn, y, mean2, rstd2, g2, d_g2, d_be2, dres=dz)
+        d_x, d_table, d_wqkv, d_bqkv, d_wproj, d_bproj = _attn_bwd32(dy, d_out.shape[:3], x2, qkv, attn, lse, table, w_qkv,
+                                                                     w_proj, ctx.geom, ctx.has_qkv_bias, dres=dy)
+        return (d_x.view(d_out.shape), d_table, d_wqkv, d_bqkv, d_wproj, d_bproj, d_g1, d_be1, d_g2, d_be2,
                 d_wfc1, d_bfc1, d_wfc2, d_bfc2, None)
 
 
@@ -450,61 +468,59 @@ class _PatchMergeFn32(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x, gamma, beta, w_red, geom):
-        from . import ops32 as o32
         H, W, eps = geom
         B, T, L, C = x.shape
-        xn, mean, rstd = o32.layernorm_fwd(x.reshape(B * T, L, C), gamma, beta, eps, patch_merge_hw=(H, W))
-        out = o32.linear(xn, w_red)
+        xn, mean, rstd = ops32.layernorm_fwd(x.reshape(B * T, L, C), gamma, beta, eps, patch_merge_hw=(H, W))
+        out = ops32.linear(xn, w_red)
         ctx.save_for_backward(x, xn, mean, rstd, gamma, w_red)
         ctx.geom = geom
         return out.view(B, T, L // 4, w_red.shape[0])
 
     @staticmethod
     def backward(ctx, d_out):
-        from . import ops32 as o32
         x, xn, mean, rstd, gamma, w_red = ctx.saved_tensors
         H, W, eps = ctx.geom
         B, T, L, C = x.shape
         d2 = d_out.contiguous().view(-1, w_red.shape[0])
-        dxn = o32.linear_dgrad(d2, w_red)
-        d_w = o32.linear_wgrad(d2, xn)
+        dxn = ops32.linear_dgrad(d2, w_red)
+        d_w = ops32.linear_wgrad(d2, xn)
         d_gamma, d_beta = _zeros_f32((4 * C,), x.device), _zeros_f32((4 * C,), x.device)
-        dx = o32.layernorm_bwd(dxn, x.reshape(B * T, L, C), mean, rstd, gamma, d_gamma, d_beta, patch_merge_hw=(H, W))
+        dx = ops32.layernorm_bwd(dxn, x.reshape(B * T, L, C), mean, rstd, gamma, d_gamma, d_beta, patch_merge_hw=(H, W))
         return dx.view(B, T, L, C), d_gamma, d_beta, d_w, None
 
 
 class _MlpFn32(torch.autograd.Function):
+    """``_MlpFn`` in the fp32-accurate mode."""
+
     @staticmethod
     def forward(ctx, x, w1, b1, w2, b2):
-        from . import ops32 as o32
         x2 = x.reshape(-1, x.shape[-1])
-        u = o32.linear(x2, w1, b1)
-        y = o32.linear(u, w2, b2, gelu_input=True)
+        u, y = _mlp_fwd32(x2, w1, b1, w2, b2)
         ctx.save_for_backward(x2, u, w1, w2)
         return y.view(*x.shape[:-1], w2.shape[0])
 
     @staticmethod
     def backward(ctx, dy):
-        from . import ops32 as o32
         x2, u, w1, w2 = ctx.saved_tensors
-        d2 = dy.contiguous().view(-1, w2.shape[0])
-        d_b2 = o32.colsum(d2, _zeros_f32((w2.shape[0],), d2.device))
-        du = o32.mul_gelu_grad(o32.linear_dgrad(d2, w2), u)
-        d_w2 = o32.linear_wgrad(d2, u, gelu_input=True)
-        d_b1 = o32.colsum(du, _zeros_f32((w1.shape[0],), d2.device))
-        return o32.linear_dgrad(du, w1).view(*dy.shape[:-1], w1.shape[1]), o32.linear_wgrad(du, x2), d_b1, d_w2, d_b2
+        dx, *grads = _mlp_bwd32(dy.contiguous().view(-1, w2.shape[0]), x2, u, w1, w2)
+        return (dx.view(*dy.shape[:-1], w1.shape[1]), *grads)
 
 
-def _as_f32(x: torch.Tensor) -> torch.Tensor:
+# The Function of each kind for the token dtype: fp32 tokens run the fp32-accurate mode.
+_ATTENTION_FNS = {_BF16: _AttentionFn, torch.float32: _AttentionFn32}
+_MLP_FNS = {_BF16: _MlpFn, torch.float32: _MlpFn32}
+_BLOCK_FNS = {_BF16: _BlockFn, torch.float32: _BlockFn32}
+_PATCH_MERGE_FNS = {_BF16: _PatchMergeFn, torch.float32: _PatchMergeFn32}
+
+
+def _in_precision(module, x: torch.Tensor, fn) -> torch.Tensor:
+    """``fn`` on x as contiguous tokens of the module's precision (fp32 in the fp32-accurate mode, else bf16), with the
+    result cast back to x's dtype."""
     if not x.is_cuda:
         raise StswinError("stswincl_b200 modules need CUDA tensors (no CPU path)")
-    return x if x.dtype == torch.float32 else x.float()
-
-
-def _as_tokens_bf16(x: torch.Tensor) -> torch.Tensor:
-    if not x.is_cuda:
-        raise StswinError("stswincl_b200 modules need CUDA tensors (no CPU path)")
-    return x if x.dtype == _BF16 else x.to(_BF16)
+    dtype = torch.float32 if _use_fp32(module, x) else _BF16
+    out = fn((x if x.dtype == dtype else x.to(dtype)).contiguous())
+    return out if out.dtype == x.dtype else out.to(x.dtype)
 
 
 class Mlp(nn.Module):
@@ -527,12 +543,8 @@ class Mlp(nn.Module):
     def forward(self, x):
         """fc1 -> GELU (erf) -> fc2 on the last dim (swin_512.py:17-23), stand-alone: two GEMMs with the bias / GELU
         epilogues fused.  Inside ``SwinTransformerBlock`` the same GEMMs run with the residual fused as well."""
-        in_dtype = x.dtype
-        if _use_fp32(self, x):
-            y = _MlpFn32.apply(_as_f32(x).contiguous(), self.fc1.weight, self.fc1.bias, self.fc2.weight, self.fc2.bias)
-            return y if in_dtype == torch.float32 else y.to(in_dtype)
-        y = _MlpFn.apply(_as_tokens_bf16(x).contiguous(), self.fc1.weight, self.fc1.bias, self.fc2.weight, self.fc2.bias)
-        return y if in_dtype == _BF16 else y.to(in_dtype)
+        params = (self.fc1.weight, self.fc1.bias, self.fc2.weight, self.fc2.bias)
+        return _in_precision(self, x, lambda t: _MLP_FNS[t.dtype].apply(t, *params))
 
 
 class WindowAttention(nn.Module):
@@ -575,14 +587,9 @@ class WindowAttention(nn.Module):
             mask = mask.detach().to(device=x_v.device, dtype=torch.float32).contiguous()
         ws = self.window_size[0]
         assert N == ws * ws and C == self.dim, "input feature has wrong size"
-        in_dtype = x_v.dtype
         geom = (ws, ws, self.num_heads, ws, 0, self._qk_scale_arg())
         args = (self.relative_position_bias_table, self.qkv.weight, self.qkv.bias, self.proj.weight, self.proj.bias, geom, mask)
-        if _use_fp32(self, x_v):
-            out = _AttentionFn32.apply(_as_f32(x_v).contiguous(), *args)
-            return out if in_dtype == torch.float32 else out.to(in_dtype)
-        out = _AttentionFn.apply(_as_tokens_bf16(x_v).contiguous(), *args)
-        return out if in_dtype == _BF16 else out.to(in_dtype)
+        return _in_precision(self, x_v, lambda t: _ATTENTION_FNS[t.dtype].apply(t, *args))
 
 
 class SwinTransformerBlock(nn.Module):
@@ -636,17 +643,13 @@ class SwinTransformerBlock(nn.Module):
         # grad mode is decided here: inside autograd.Function.forward it always reads "disabled", and
         # ctx.needs_input_grad ignores torch.no_grad()
         infer = not torch.is_grad_enabled()
-        fn = _BlockFn32 if x.dtype == torch.float32 else _BlockFn          # fp32 tokens: the fp32-accurate mode
-        return fn.apply(x, *self._block_params(), self._geom() + (infer,))
+        return _BLOCK_FNS[x.dtype].apply(x, *self._block_params(), self._geom() + (infer,))
 
     def forward(self, x_v):
         H, W = self.input_resolution
         B, T, L, C = x_v.shape
         assert L == H * W, "input feature has wrong size"
-        in_dtype = x_v.dtype
-        tokens = _as_f32(x_v) if _use_fp32(self, x_v) else _as_tokens_bf16(x_v)
-        out = self.forward_tokens(tokens.contiguous())
-        return out if in_dtype == out.dtype else out.to(in_dtype)
+        return _in_precision(self, x_v, self.forward_tokens)
 
 
 class PatchMerging(nn.Module):
@@ -661,18 +664,14 @@ class PatchMerging(nn.Module):
 
     def forward_tokens(self, x: torch.Tensor) -> torch.Tensor:
         H, W = self.input_resolution
-        fn = _PatchMergeFn32 if x.dtype == torch.float32 else _PatchMergeFn
-        return fn.apply(x, self.norm.weight, self.norm.bias, self.reduction.weight, (H, W, self.norm.eps))
+        return _PATCH_MERGE_FNS[x.dtype].apply(x, self.norm.weight, self.norm.bias, self.reduction.weight, (H, W, self.norm.eps))
 
     def forward(self, x):
         H, W = self.input_resolution
         B, T, L, C = x.shape
         assert L == H * W, "input feature has wrong size"
         assert H % 2 == 0 and W % 2 == 0, f"x size ({H}*{W}) are not even."
-        in_dtype = x.dtype
-        tokens = _as_f32(x) if _use_fp32(self, x) else _as_tokens_bf16(x)
-        out = self.forward_tokens(tokens.contiguous())
-        return out if in_dtype == out.dtype else out.to(in_dtype)
+        return _in_precision(self, x, self.forward_tokens)
 
 
 class SwinTransformerLayerv5(nn.Module):
@@ -710,13 +709,7 @@ class SwinTransformerLayerv5(nn.Module):
             y = blk1.forward_tokens(blk0.forward_tokens(x.view(B * 2, 2, L, C)))
             return y.view(B, 4, L, C)
         if not torch.is_grad_enabled():
-            xm = torch.empty((B, 2, L, C), dtype=x.dtype, device=x.device)
-            ops.copy_frames(xm, x[:, 1:3])
-            out = torch.empty_like(x)
-            ops.copy_frames(out[:, 0], x[:, 0])
-            ops.copy_frames(out[:, 3], x[:, 3])
-            ops.copy_frames(out[:, 1:3], blk1.forward_tokens(blk0.forward_tokens(xm)))
-            return out
+            return _mid_frames(x, lambda xm: blk1.forward_tokens(blk0.forward_tokens(xm)))
         return _MidLayerFn.apply(x, blk0._geom() + (False,), blk1._geom() + (False,), *blk0._block_params(), *blk1._block_params())
 
     def _check_input(self, x_v):

@@ -144,6 +144,30 @@ def test_standalone_window_attention_with_dense_mask_fp32():
         assert rel_err(p.grad.cpu(), leaf[n].grad) < TOL, n
 
 
+def test_standalone_mlp_fp32_vs_oracle():
+    """Mlp.forward (swin_512.py:17-23) on its own in the fp32-accurate mode, forward + backward, against the CPU oracle."""
+    from oracle import swin_oracle as so
+    from stswincl_b200 import swin
+    gen = torch.Generator().manual_seed(3)
+    params = {"fc1.weight": torch.randn(512, 128, generator=gen) * 128 ** -0.5, "fc1.bias": 0.5 * torch.randn(512, generator=gen),
+              "fc2.weight": torch.randn(128, 512, generator=gen) * 512 ** -0.5, "fc2.bias": 0.5 * torch.randn(128, generator=gen)}
+    m = _load(swin.Mlp(128, 512), params)
+    x = torch.randn(2, 50, 128, generator=gen)
+    wgt = torch.randn(2, 50, 128, generator=gen)
+    leaf = {k: v.clone().requires_grad_(True) for k, v in params.items()}
+    xr = x.clone().requires_grad_(True)
+    ref = so.mlp(xr, leaf)
+    (ref * wgt).sum().backward()
+    xg = x.cuda().requires_grad_(True)
+    y = m(xg)
+    assert y.dtype == torch.float32 and y.shape == ref.shape
+    (y * wgt.cuda()).sum().backward()
+    torch.cuda.synchronize()
+    assert rel_err(y.cpu(), ref) < TOL and rel_err(xg.grad.cpu(), xr.grad) < TOL
+    for n, p in m.named_parameters():
+        assert rel_err(p.grad.cpu(), leaf[n].grad) < TOL, n
+
+
 def test_precision_auto_follows_the_input_dtype():
     from oracle import swin_oracle as so
     from stswincl_b200 import swin

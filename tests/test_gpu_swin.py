@@ -259,6 +259,36 @@ def test_standalone_mlp_forward_backward():
         assert rel_err(p.grad, g) < 2e-2
 
 
+@pytest.mark.parametrize("precision,tol", [("bf16", TOL), ("fp32", 1e-3)])
+def test_standalone_patch_merging_vs_oracle(precision, tol):
+    """PatchMerging.forward (swin_512.py:255-277) called on its own, forward + backward, against the CPU oracle in both
+    precisions (the bf16 mode's input is rounded to bf16 for the oracle too)."""
+    from oracle import swin_oracle as so
+    from stswincl_b200 import swin
+    dim, (H, W) = 128, (16, 24)
+    gen = torch.Generator().manual_seed(7)
+    params = {"reduction.weight": torch.randn(2 * dim, 4 * dim, generator=gen) * (4 * dim) ** -0.5,
+              "norm.weight": 1.0 + 0.2 * torch.randn(4 * dim, generator=gen), "norm.bias": 0.2 * torch.randn(4 * dim, generator=gen)}
+    m = _load(swin.PatchMerging((H, W), dim), params)
+    m.precision = precision
+    x = so.make_features(8, 2, 2, H * W, dim)
+    if precision == "bf16":
+        x = x.to(torch.bfloat16).float()
+    wgt = torch.randn(2, 2, H * W // 4, 2 * dim, generator=gen)
+    leaf = {k: v.clone().requires_grad_(True) for k, v in params.items()}
+    xr = x.clone().requires_grad_(True)
+    ref = so.patch_merging(xr, leaf, (H, W))
+    (ref * wgt).sum().backward()
+    xg = x.cuda().requires_grad_(True)
+    y = m(xg)
+    assert y.dtype == torch.float32 and y.shape == ref.shape
+    (y * wgt.cuda()).sum().backward()
+    torch.cuda.synchronize()
+    assert rel_err(y.cpu(), ref) < tol and rel_err(xg.grad.cpu(), xr.grad) < tol
+    for n, p in m.named_parameters():
+        assert rel_err(p.grad.cpu(), leaf[n].grad) < tol, n
+
+
 def test_layer_dtype_contract_fp16_and_autocast():
     """The reference's layer returns its input dtype (:326); under amp.autocast its last op (LayerNorm) returns fp32."""
     from stswincl_b200 import swin
