@@ -278,6 +278,24 @@ int stswin_adam_step(void* const* params, const void* const* grads, void* const*
                      void* const* shadows, const int64_t* numels, int n_tensors, int grads_are_bf16, float lr, float beta1,
                      float beta2, float eps, float weight_decay, float grad_scale, float* step, void* stream);
 
+/* torch.optim.SGD step over a list of tensors (the optimiser of the fine-tune recipe train_CL_ft_mswin_sgd_minput.py),
+ * emitting the bf16 copy of the updated weights like stswin_adam_step.  Per element:
+ *   g = grad_scale * grad;  g = maximize ? -g : g;  g = g + weight_decay * p (when weight_decay != 0);
+ *   when momentum != 0: buf = first_step[t] ? g : momentum * buf + one_minus_dampening * g;
+ *                       d = nesterov ? g + momentum * buf : buf   (else d = g);
+ *   p = p - lr * d;  shadow = bf16(p)
+ * Each operation is rounded as in torch's single-tensor step (one fma per add(alpha=), one product per mul_), so the
+ * result is bit-identical with it; p.grad is not written.  one_minus_dampening is passed, not computed, so that the
+ * caller rounds the same (double) 1 - dampening torch does.  lr: the host value, or *lr_dev when lr_dev (a device fp32
+ * scalar) is non-NULL -- a captured step then follows a schedule that rewrites the scalar between replays.
+ * params / momentum_bufs: fp32; grads: fp32, or bf16 when grads_are_bf16; shadows: bf16 or NULL (whole array or per
+ * tensor); momentum_bufs may be NULL when momentum == 0; first_step: non-zero for a tensor without a momentum buffer
+ * yet (NULL: none).  All tables are HOST arrays of n_tensors entries; one launch per 48 tensors. */
+int stswin_sgd_step(void* const* params, const void* const* grads, void* const* momentum_bufs, void* const* shadows,
+                    const int64_t* numels, const uint8_t* first_step, int n_tensors, int grads_are_bf16, float lr,
+                    const float* lr_dev, float momentum, float one_minus_dampening, int nesterov, int maximize,
+                    float weight_decay, float grad_scale, void* stream);
+
 /* dst[t] = cast(src[t]) over a list of fp32 tensors (HOST arrays of n_tensors device pointers / element counts):
  * gathers the gradients a backward segment produced into the flat bucket of the data-parallel all-reduce (SURVEY.md
  * section 8e, C1), rounding to bf16 when dst_is_bf16 (bytes on the wire halved) -- one launch per 48 tensors. */

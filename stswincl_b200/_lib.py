@@ -98,6 +98,8 @@ SIGNATURES = {
     "stswin_lars_sgd_step": ([_vp, _vp, _vp, _vp, _vp, _i] + [ctypes.c_float] * 3 + [_i, ctypes.c_float, _i,
                              ctypes.c_float, ctypes.c_float, _vp, _vp], ctypes.c_int),
     "stswin_adam_step": ([_vp] * 6 + [_i, _i] + [ctypes.c_float] * 6 + [_vp, _vp], ctypes.c_int),
+    "stswin_sgd_step": ([_vp] * 6 + [_i, _i, ctypes.c_float, _fp] + [ctypes.c_float] * 2 + [_i, _i] + [ctypes.c_float] * 2
+                        + [_vp], ctypes.c_int),
     "stswin_gather_cast": ([_vp, _vp, _vp, _i, _i, _vp], ctypes.c_int),
     "stswin_f32_split": ([_vp, _vp, _i64, _i, _i, _i, _i, _vp], ctypes.c_int),
     "stswin_f32_rowop": ([_vp, _vp, _vp, _vp, _i64, _i, _i, _vp], ctypes.c_int),

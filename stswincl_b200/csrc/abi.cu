@@ -5,7 +5,7 @@
 
 extern "C" {
 
-int stswin_abi_version(void) { return 4; }
+int stswin_abi_version(void) { return 5; }
 const char* stswin_last_error(void) { return stswin::last_error(); }
 int stswin_set_device(int device) {
   STSWIN_CUDA(cudaSetDevice(device));
@@ -116,6 +116,15 @@ int stswin_adam_step(void* const* params, const void* const* grads, void* const*
                      float beta2, float eps, float weight_decay, float grad_scale, float* step, void* stream) {
   return stswin::adam_step(params, grads, exp_avg, exp_avg_sq, shadows, numels, n_tensors, grads_are_bf16, lr, beta1, beta2,
                            eps, weight_decay, grad_scale, step, static_cast<cudaStream_t>(stream));
+}
+
+int stswin_sgd_step(void* const* params, const void* const* grads, void* const* momentum_bufs, void* const* shadows,
+                    const int64_t* numels, const uint8_t* first_step, int n_tensors, int grads_are_bf16, float lr,
+                    const float* lr_dev, float momentum, float one_minus_dampening, int nesterov, int maximize,
+                    float weight_decay, float grad_scale, void* stream) {
+  return stswin::sgd_step(params, grads, momentum_bufs, shadows, numels, first_step, n_tensors, grads_are_bf16, lr, lr_dev,
+                          momentum, one_minus_dampening, nesterov, maximize, weight_decay, grad_scale,
+                          static_cast<cudaStream_t>(stream));
 }
 
 int stswin_gather_cast(void* const* dst, const void* const* src, const int64_t* numels, int n_tensors, int dst_is_bf16,

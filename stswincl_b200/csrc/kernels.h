@@ -55,6 +55,10 @@ int lars_sgd_step(void* const* params, void* const* grads, void* const* bufs, co
 int adam_step(void* const* params, const void* const* grads, void* const* exp_avg, void* const* exp_avg_sq,
               void* const* shadows, const int64_t* numels, int n_tensors, int grads_are_bf16, float lr, float beta1,
               float beta2, float eps, float weight_decay, float grad_scale, float* step, cudaStream_t stream);
+int sgd_step(void* const* params, const void* const* grads, void* const* momentum_bufs, void* const* shadows,
+             const int64_t* numels, const uint8_t* first_step, int n_tensors, int grads_are_bf16, float lr, const float* lr_dev,
+             float momentum, float one_minus_dampening, int nesterov, int maximize, float weight_decay, float grad_scale,
+             cudaStream_t stream);
 int gather_cast(void* const* dst, const void* const* src, const int64_t* numels, int n_tensors, int dst_is_bf16,
                 cudaStream_t stream);
 

@@ -381,7 +381,8 @@ struct MtArgs {
   int n;
 };
 
-__device__ __forceinline__ int mt_find(const MtArgs& t, int block) {
+template <class Args>
+__device__ __forceinline__ int mt_find(const Args& t, int block) {
   int lo = 0, hi = t.n - 1;
   while (lo < hi) {
     const int mid = (lo + hi + 1) >> 1;
@@ -615,6 +616,88 @@ __global__ void __launch_bounds__(kThreads) adam_kernel(const __grid_constant__ 
   }
 }
 
+// ------------------------------------------------------------------------------------------------
+// torch.optim.SGD (momentum, dampening, nesterov, weight decay, maximize) as a multi-tensor stream that also emits the
+// bf16 shadow of the weights.  Each operation is rounded where the eager single-tensor step of torch rounds it --
+// add(alpha=) is one fma of alpha * other onto self, mul_ one product, every eager op its own rounding -- so the result
+// is bit-identical with it and does not depend on the compiler's contraction choices.  p.grad is not written.
+struct SgdStepArgs {
+  float* p[MT_MAX];
+  const void* g[MT_MAX];
+  float* buf[MT_MAX];                // momentum buffers; all null when momentum == 0
+  __nv_bfloat16* shadow[MT_MAX];     // may be null per tensor
+  long numel[MT_MAX];
+  int block_start[MT_MAX + 1];
+  unsigned char first[MT_MAX];       // the tensor's first step with momentum: buf = g
+  int n;
+  int grad_bf16, nesterov, maximize;
+  float lr, momentum, one_minus_dampening, wd, grad_scale;
+  const float* lr_dev;               // device scalar read instead of lr when non-null (a schedule under graph replay)
+};
+
+__global__ void __launch_bounds__(kThreads) sgd_kernel(const __grid_constant__ SgdStepArgs t) {
+  pdl_wait();
+  pdl_launch_dependents();
+  const int ti = mt_find(t, blockIdx.x);
+  float* __restrict__ p = t.p[ti];
+  float* __restrict__ buf = t.buf[ti];
+  __nv_bfloat16* __restrict__ sh = t.shadow[ti];
+  const void* gp = t.g[ti];
+  const bool has_buf = t.momentum != 0.f, first = t.first[ti] != 0;
+  const long n = t.numel[ti];
+  const long base = (long)(blockIdx.x - t.block_start[ti]) * MT_CHUNK;
+  const long end = base + MT_CHUNK < n ? base + MT_CHUNK : n;
+  const float neg_lr = -(t.lr_dev != nullptr ? __ldg(t.lr_dev) : t.lr);
+  auto one = [&](float pv, float gv, float& bv) -> float {
+    float g = __fmul_rn(gv, t.grad_scale);
+    if (t.maximize) g = -g;
+    if (t.wd != 0.f) g = __fmaf_rn(t.wd, pv, g);                                    // grad.add(param, alpha=wd)
+    float d = g;
+    if (has_buf) {
+      bv = first ? g : __fmaf_rn(t.one_minus_dampening, g, __fmul_rn(bv, t.momentum));  // buf.mul_(m).add_(g, alpha=1-damp)
+      d = t.nesterov ? __fmaf_rn(t.momentum, bv, g) : bv;                          // grad.add(buf, alpha=m)
+    }
+    return __fmaf_rn(neg_lr, d, pv);                                                // param.add_(d, alpha=-lr)
+  };
+  const bool al = ((((uintptr_t)p | (uintptr_t)buf) & 15) == 0) && ((((uintptr_t)gp) & (t.grad_bf16 ? 7 : 15)) == 0) &&
+                  ((((uintptr_t)sh) & 7) == 0);
+  long i;
+  if (al) {
+    const long end4 = base + ((end - base) & ~3L);
+#pragma unroll 2
+    for (i = base + threadIdx.x * 4; i < end4; i += kThreads * 4) {
+      float4 pv = *reinterpret_cast<const float4*>(p + i);
+      float4 gv;
+      if (t.grad_bf16) {
+        const uint2 raw = __ldg(reinterpret_cast<const uint2*>(static_cast<const __nv_bfloat16*>(gp) + i));
+        const float2 a = unpack_bf16(raw.x), b = unpack_bf16(raw.y);
+        gv = make_float4(a.x, a.y, b.x, b.y);
+      } else {
+        gv = __ldg(reinterpret_cast<const float4*>(static_cast<const float*>(gp) + i));
+      }
+      float4 bv = (has_buf && !first) ? *reinterpret_cast<const float4*>(buf + i) : make_float4(0.f, 0.f, 0.f, 0.f);
+      pv.x = one(pv.x, gv.x, bv.x);
+      pv.y = one(pv.y, gv.y, bv.y);
+      pv.z = one(pv.z, gv.z, bv.z);
+      pv.w = one(pv.w, gv.w, bv.w);
+      *reinterpret_cast<float4*>(p + i) = pv;
+      if (has_buf) *reinterpret_cast<float4*>(buf + i) = bv;
+      if (sh != nullptr) *reinterpret_cast<uint2*>(sh + i) = make_uint2(pack_bf16(pv.x, pv.y), pack_bf16(pv.z, pv.w));
+    }
+    i = end4 + threadIdx.x;
+  } else {
+    i = base + threadIdx.x;
+  }
+  for (; i < end; i += kThreads) {
+    const float gv = t.grad_bf16 ? __bfloat162float(static_cast<const __nv_bfloat16*>(gp)[i]) : static_cast<const float*>(gp)[i];
+    float bv = (has_buf && !first) ? buf[i] : 0.f;
+    const float pv = one(p[i], gv, bv);
+    p[i] = pv;
+    if (has_buf) buf[i] = bv;
+    if (sh != nullptr) sh[i] = __float2bfloat16_rn(pv);
+  }
+}
+
 // dst[t] = cast(src[t]) for a list of fp32 tensors: gathers the gradients of a backward segment into the flat
 // bucket a data-parallel all-reduce sends (bf16 on the wire, or fp32)
 __global__ void __launch_bounds__(kThreads) mt_gather_kernel(const __grid_constant__ MtArgs t, int to_bf16) {
@@ -780,6 +863,43 @@ int adam_step(void* const* params, const void* const* grads, void* const* exp_av
     a.grad_scale = grad_scale; a.step = step;
     if (blocks == 0) continue;
     STSWIN_CUDA(launch_pdl(adam_kernel, dim3(blocks), dim3(kThreads), 0, stream, a));
+  }
+  STSWIN_CUDA(cudaGetLastError());
+  return kOk;
+}
+
+int sgd_step(void* const* params, const void* const* grads, void* const* momentum_bufs, void* const* shadows,
+             const int64_t* numels, const uint8_t* first_step, int n_tensors, int grads_are_bf16, float lr, const float* lr_dev,
+             float momentum, float one_minus_dampening, int nesterov, int maximize, float weight_decay, float grad_scale,
+             cudaStream_t stream) {
+  STSWIN_CHECK_ARG(n_tensors >= 0 && (n_tensors == 0 || (params && grads && numels)), "sgd_step: null table");
+  STSWIN_CHECK_ARG(momentum == 0.f || momentum_bufs != nullptr, "sgd_step: momentum needs momentum buffers");
+  STSWIN_CHECK_ARG(!nesterov || (momentum > 0.f && one_minus_dampening == 1.f),
+                   "sgd_step: nesterov needs momentum and zero dampening");
+  if (n_tensors == 0) return kOk;
+  for (int t0 = 0; t0 < n_tensors; t0 += MT_MAX) {
+    SgdStepArgs a;
+    const int cnt = n_tensors - t0 < MT_MAX ? n_tensors - t0 : MT_MAX;
+    int blocks = 0;
+    a.n = cnt;
+    for (int i = 0; i < cnt; ++i) {
+      STSWIN_CHECK_ARG(params[t0 + i] && grads[t0 + i] && (momentum == 0.f || momentum_bufs[t0 + i]),
+                       "sgd_step: null tensor %d", t0 + i);
+      a.p[i] = static_cast<float*>(params[t0 + i]);
+      a.g[i] = grads[t0 + i];
+      a.buf[i] = momentum != 0.f ? static_cast<float*>(momentum_bufs[t0 + i]) : nullptr;
+      a.shadow[i] = shadows ? static_cast<__nv_bfloat16*>(shadows[t0 + i]) : nullptr;
+      a.numel[i] = numels[t0 + i];
+      a.first[i] = first_step ? first_step[t0 + i] : 0;
+      a.block_start[i] = blocks;
+      blocks += (int)((numels[t0 + i] + MT_CHUNK - 1) / MT_CHUNK);
+    }
+    a.block_start[cnt] = blocks;
+    a.grad_bf16 = grads_are_bf16; a.nesterov = nesterov; a.maximize = maximize;
+    a.lr = lr; a.momentum = momentum; a.one_minus_dampening = one_minus_dampening; a.wd = weight_decay;
+    a.grad_scale = grad_scale; a.lr_dev = lr_dev;
+    if (blocks == 0) continue;
+    STSWIN_CUDA(launch_pdl(sgd_kernel, dim3(blocks), dim3(kThreads), 0, stream, a));
   }
   STSWIN_CUDA(cudaGetLastError());
   return kOk;

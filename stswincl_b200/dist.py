@@ -10,6 +10,7 @@ These helpers are backend-agnostic (NCCL on GPUs, gloo in the CPU tests).
 """
 from __future__ import annotations
 
+import inspect
 from typing import Iterable, List, Optional, Sequence
 
 import torch
@@ -104,6 +105,15 @@ class FlatGradients:
             p.grad = v
 
 
+def _takes_grads(opt) -> bool:
+    """Whether ``opt.step`` accepts ``grads=``.  Read through the signature: ``torch.optim.Optimizer`` wraps ``step``
+    in a ``(*args, **kwargs)`` profiling wrapper, whose own code object does not name the parameter."""
+    try:
+        return "grads" in inspect.signature(opt.step).parameters
+    except (AttributeError, TypeError, ValueError):
+        return False
+
+
 class SegmentedStep:
     """Data-parallel training step whose gradient exchange overlaps the backward.
 
@@ -116,7 +126,7 @@ class SegmentedStep:
     optimizer step are issued between / after the replays.
 
     The optimizer step reads the reduced gradients straight from the buckets when the optimizer accepts
-    ``step(grads=...)`` (``optim.FusedAdam``: fp32 or bf16 gradients); otherwise they are copied back into
+    ``step(grads=...)`` (``optim.FusedAdam``, ``optim.FusedSGD``: fp32 or bf16 gradients); otherwise they are copied back into
     ``p.grad`` first.  Backend-agnostic (NCCL on GPUs, gloo in the CPU tests; there ``use_graph=False``)."""
 
     def __init__(self, model, optimizer, loss_fn, *, segments: int = 4, wire_dtype: torch.dtype = torch.bfloat16,
@@ -157,7 +167,7 @@ class SegmentedStep:
             self._buckets.append(buf)
             self._views.append(views)
         self._view_of = {id(p): v for ps, vs in zip(self._stage_params, self._views) for p, v in zip(ps, vs)}
-        self._direct = hasattr(self.opt, "step") and "grads" in getattr(self.opt.step, "__code__", type("c", (), {"co_varnames": ()})).co_varnames
+        self._direct = _takes_grads(self.opt)
         self._opt_grads = [self._view_of[id(p)] for g in self.opt.param_groups for p in g["params"] if p.requires_grad]
         self._cuda = dev.type == "cuda"
         if self._cuda:

@@ -1,5 +1,11 @@
-"""Drop-in replacements for the optimiser-side loops of the pre-training caller (SURVEY.md section 8f, N2 / N4).
+"""Drop-in replacements for the optimiser-side loops of the STswinCL training recipes (SURVEY.md section 8f, N2 / N4).
 
+  * ``FusedAdam``                    -- ``torch.optim.Adam`` of ``seg18/train_swin.py``: multi-tensor, reads fp32 or bf16
+    (all-reduce bucket) gradients, writes the bf16 shadow of the weights the Swin kernels read (``bf16_weight``).
+  * ``FusedSGD``                     -- ``torch.optim.SGD`` of the fine-tune recipe
+    ``train_CL_ft_mswin_sgd_minput.py:147-162`` (momentum, per-module groups, poly lr): the same contract as
+    ``FusedAdam``, bit-identical with torch's single-tensor step, ``state_dict`` compatible with ``torch.optim.SGD``, and
+    a device-tensor ``lr`` that a CUDA-graph-captured step reads on every replay.
   * ``LARS`` / ``add_weight_decay``  -- ``pixcontrast_18/contrast/lars.py`` (same names, constructor, wrapper
     semantics: ``LARS(torch.optim.SGD(add_weight_decay(model, wd), lr, momentum))``).  The reference calls
     ``p.norm()`` / ``p.grad.norm()`` per tensor and branches on the results in Python (:127-133), a host
@@ -23,7 +29,7 @@ from torch.optim.optimizer import Optimizer
 from . import _lib, ops
 from ._lib import StswinError
 
-__all__ = ["LARS", "FusedAdam", "add_weight_decay", "momentum_update", "bf16_weight"]
+__all__ = ["LARS", "FusedAdam", "FusedSGD", "add_weight_decay", "momentum_update", "bf16_weight"]
 
 
 def add_weight_decay(model, weight_decay=1e-5, skip_list=()):
@@ -168,8 +174,8 @@ class LARS(Optimizer):
 # bf16 shadow of the weights
 # ---------------------------------------------------------------------------------------------------------------
 def bf16_weight(w: torch.Tensor) -> torch.Tensor:
-    """The bf16 copy of a weight the GEMM kernels consume.  ``FusedAdam`` keeps a shadow copy per parameter that its
-    update kernel rewrites every step, so the forward needs no cast kernel; the shadow is valid as long as nobody else
+    """The bf16 copy of a weight the GEMM kernels consume.  ``FusedAdam`` and ``FusedSGD`` keep a shadow copy per
+    parameter that their update kernel rewrites every step, so the forward needs no cast kernel; the shadow is valid as long as nobody else
     wrote the parameter (tracked by the tensor's version counter -- the kernel does not bump it).  Without a valid
     shadow this is ``w.to(bfloat16)``."""
     sh = getattr(w, "_stswin_shadow", None)
@@ -249,4 +255,122 @@ class FusedAdam(Optimizer):
                                           ops._stream(params[0]))
             _lib.check(st, "stswin_adam_step")
             ops.count_extra_launches((len(params) + 31) // 32)
+        return loss
+
+
+def _shadow_ptr(p: torch.Tensor, enabled: bool):
+    """The bf16 shadow of ``p`` that an update kernel rewrites (created for >= 2-D weights when ``enabled``), or None."""
+    sh = getattr(p, "_stswin_shadow", None)
+    if sh is None or sh[0].device != p.device:
+        if not enabled or p.dim() < 2:
+            return None
+        sh = p._stswin_shadow = (p.detach().to(torch.bfloat16), p._version)
+    elif sh[1] != p._version:                      # stale shadow: the kernel rewrites it anyway
+        sh = p._stswin_shadow = (sh[0], p._version)
+    return sh[0].data_ptr()
+
+
+class FusedSGD(Optimizer):
+    """``torch.optim.SGD`` (momentum, dampening, nesterov, weight decay, maximize) as multi-tensor launches of
+    ``stswin_sgd_step`` (48 tensors per launch), bit-identical with torch's single-tensor step, that also write the bf16
+    shadow of every >= 2-D weight in the same pass (``bf16_weight``).  State is ``state[p]["momentum_buffer"]`` as in
+    torch, so ``state_dict`` / ``load_state_dict`` interoperate with ``torch.optim.SGD`` both ways.  ``foreach`` /
+    ``fused`` are accepted and ignored.
+
+    ``lr`` may be a 0-dim fp32 CUDA tensor: the kernel reads it on the device, so a CUDA-graph-captured step follows a
+    schedule that writes the tensor between replays.  The step is capturable once every parameter with momentum has a
+    buffer (after one eager step), as for torch's SGD.
+
+    ``step(grads=...)`` takes the gradients from a list (fp32 or bf16, one per ``requires_grad`` parameter in group
+    order) instead of ``p.grad``, scaled by ``grad_scale`` -- the bf16 bucket views of a data-parallel all-reduce
+    (``dist.SegmentedStep``).  ``p.grad`` is never written."""
+
+    def __init__(self, params, lr=1e-3, momentum=0, dampening=0, weight_decay=0, nesterov=False, *, maximize=False,
+                 foreach=None, differentiable=False, fused=None, shadow: bool = True):
+        if isinstance(lr, torch.Tensor) and lr.numel() != 1:
+            raise ValueError("Tensor lr must be 1-element")
+        if lr < 0.0:
+            raise ValueError(f"Invalid learning rate: {lr}")
+        if momentum < 0.0:
+            raise ValueError(f"Invalid momentum value: {momentum}")
+        if weight_decay < 0.0:
+            raise ValueError(f"Invalid weight_decay value: {weight_decay}")
+        if nesterov and (momentum <= 0 or dampening != 0):
+            raise ValueError("Nesterov momentum requires a momentum and zero dampening")
+        if differentiable:
+            raise StswinError("FusedSGD: differentiable=True is not supported (the update runs in a CUDA kernel)")
+        # foreach / fused are kept in the groups (unused here) so that a torch.optim.SGD loading this state takes them
+        super().__init__(params, dict(lr=lr, momentum=momentum, dampening=dampening, weight_decay=weight_decay,
+                                      nesterov=nesterov, maximize=maximize, foreach=foreach, differentiable=False,
+                                      fused=fused))
+        self.shadow = shadow
+
+    def __setstate__(self, state):
+        super().__setstate__(state)
+        for group in self.param_groups:
+            group.setdefault("nesterov", False)
+            group.setdefault("maximize", False)
+
+    @staticmethod
+    def _lr(lr, dev):
+        """(host lr, device lr pointer) of a group's ``lr``."""
+        if not torch.is_tensor(lr):
+            return float(lr), None
+        if lr.dim() != 0 or lr.dtype != torch.float32 or lr.device != dev:
+            raise StswinError(f"FusedSGD.step: a tensor lr must be a 0-dim fp32 tensor on {dev}, got {lr.dtype} "
+                              f"{tuple(lr.shape)} on {lr.device}")
+        return 0.0, lr.data_ptr()
+
+    @torch.no_grad()
+    def step(self, closure=None, grads=None, grad_scale: float = 1.0):
+        loss = None
+        if closure is not None:
+            with torch.enable_grad():
+                loss = closure()
+        lib = _lib.load()
+        gi = 0
+        for group in self.param_groups:
+            if grads is None:
+                params = [p for p in group["params"] if p.grad is not None]
+                gl = [p.grad for p in params]
+            else:
+                params = [p for p in group["params"] if p.requires_grad]
+                gl = list(grads[gi:gi + len(params)])
+                gi += len(params)
+            if not params:
+                continue
+            _check_f32(params, "FusedSGD.step")
+            if any(g.is_sparse for g in gl):
+                raise StswinError("FusedSGD.step: sparse gradients are not supported")
+            gdt = gl[0].dtype
+            if gdt not in (torch.float32, torch.bfloat16) or any(g.dtype != gdt or not g.is_contiguous() or not g.is_cuda or
+                                                                 g.numel() != p.numel() for g, p in zip(gl, params)):
+                raise StswinError("FusedSGD.step: gradients must be contiguous CUDA tensors, all fp32 or all bf16, one per "
+                                  "parameter and of its size")
+            lr, lr_dev = self._lr(group["lr"], params[0].device)
+            momentum = float(group["momentum"])
+            bufs, first = None, None
+            if momentum != 0:
+                bufs, flags = [], []
+                for p in params:
+                    st = self.state[p]
+                    buf = st.get("momentum_buffer")
+                    flags.append(1 if buf is None else 0)
+                    if buf is None:
+                        buf = st["momentum_buffer"] = torch.zeros_like(p, memory_format=torch.contiguous_format)
+                    bufs.append(buf)
+                _check_f32(bufs, "FusedSGD.step (momentum_buffer)")
+                first = (ctypes.c_uint8 * len(flags))(*flags)
+            shadows = [_shadow_ptr(p, self.shadow) for p in params]
+            n_el = sum(p.numel() for p in params)
+            n_bytes = n_el * (8 + gl[0].element_size() + (8 if bufs else 0)) + \
+                sum(p.numel() for p, s in zip(params, shadows) if s is not None) * 2
+            with ops._launch("sgd_step", float(n_bytes), params[0]):
+                st = lib.stswin_sgd_step(_ptrs(params), _ptrs(gl), _ptrs(bufs) if bufs else None,
+                                         (ctypes.c_void_p * len(shadows))(*shadows), _numels(params), first, len(params),
+                                         int(gdt == torch.bfloat16), lr, lr_dev, momentum, float(1 - group["dampening"]),
+                                         int(bool(group["nesterov"])), int(bool(group["maximize"])),
+                                         float(group["weight_decay"]), float(grad_scale), ops._stream(params[0]))
+            _lib.check(st, "stswin_sgd_step")
+            ops.count_extra_launches((len(params) + 47) // 48 - 1)
         return loss
