@@ -247,24 +247,37 @@ int stswin_ohem_ce_bwd(const void* logits, int logits_is_f32, const int64_t* lab
 
 /* Momentum (EMA) update of the key encoder as one multi-tensor stream.  Replaces the ~600 per-parameter
  * `param_k.data = param_k.data * m + param_q.data * (1. - m)` of PixPro._momentum_update_key_encoder
- * (pixcontrast_18/contrast/models/PixPro_swin_v5.py:258-289); bit-exact with the eager expression
- * (two rounded products, one rounded sum).  k_params / q_params / numels are HOST arrays of n_tensors
- * device pointers (fp32 tensors, contiguous) and element counts. */
-int stswin_ema_update(void* const* k_params, const void* const* q_params, const int64_t* numels, int n_tensors, float m,
-                      float one_minus_m, void* stream);
+ * (pixcontrast_18/contrast/models/PixPro_swin_v5.py:258-289).  Per element:
+ *   k = rn(rn(k * m) + rn(q * one_minus_m));  k_shadow = bf16_rn(k)
+ * i.e. bit-exact with the eager expression (two rounded products, one rounded sum) when m and one_minus_m are the fp32
+ * roundings of the double m and 1. - m that the expression rounds.  (m, one_minus_m) are the host values, or m_dev[0],
+ * m_dev[1] when m_dev (a device fp32 pair) is non-NULL -- a captured update then follows a schedule that rewrites the
+ * pair between replays.  k_params / q_params / k_shadows / numels are HOST arrays of n_tensors device pointers (fp32
+ * tensors, contiguous; k_shadows: bf16 or NULL, whole array or per tensor) and element counts. */
+int stswin_ema_update(void* const* k_params, const void* const* q_params, void* const* k_shadows, const int64_t* numels,
+                      int n_tensors, float m, float one_minus_m, const float* m_dev, void* stream);
 
 /* LARS-scaled SGD step of one parameter group.  Replaces LARS.apply_adaptive_lrs + the wrapped
- * torch.optim.SGD.step (pixcontrast_18/contrast/lars.py:109-152): per tensor
- *   g = grad + weight_decay * p (:121-122); if `lars`: g *= trust_coef * |p| / (|g| + eps) when both norms
- *   are positive (:125-135); grad <- g (the reference rebinds p.grad); buf = g on a tensor's first step
- *   (first_step[t] != 0) else momentum * buf + (1 - dampening) * g; p -= lr * (nesterov ? g + momentum * buf : buf).
- * The norms are reduced on the device (no .norm() host reads, :127-133).  params / grads / momentum_bufs /
- * numels / first_step are HOST arrays over the group's tensors (fp32, contiguous); momentum_bufs may be NULL
- * when momentum == 0; norms_ws: device [2 * n_tensors] fp64 scratch (only when `lars`). */
-int stswin_lars_sgd_step(void* const* params, void* const* grads, void* const* momentum_bufs, const int64_t* numels,
-                         const uint8_t* first_step, int n_tensors, float lr, float momentum, float dampening,
-                         int nesterov, float weight_decay, int lars, float trust_coef, float eps, double* norms_ws,
-                         void* stream);
+ * torch.optim.SGD.step (pixcontrast_18/contrast/lars.py:109-152).  Per tensor, with the norms reduced on the device
+ * (fp64 sums of fp32 block partials; no .norm() host reads, :127-133):
+ *   g = fma(weight_decay, p, grad) when weight_decay > 0 (:121-122);
+ *   if `lars` and |p| > 0 and |g| > 0: g = rn(g * rn(rn(trust_coef * |p|) / rn(|g| + eps))) (:125-135);
+ *   grad <- g when write_grads (the reference rebinds p.grad);
+ *   when momentum != 0: buf = first_step[t] ? g : fma(1 - dampening, g, rn(momentum * buf)) where the tensor's
+ *                       16-byte path runs, fma(momentum, buf, rn((1 - dampening) * g)) on its scalar tail and when
+ *                       a pointer is not 16-byte aligned (the roundings of ABI version 5, kept bit for bit);
+ *                       d = nesterov ? fma(momentum, buf, g) : buf   (else d = g);
+ *   p = fma(-lr, d, p);  shadow = bf16_rn(p)
+ * lr: the host value, or *lr_dev when lr_dev (a device fp32 scalar) is non-NULL -- a captured step then follows a
+ * schedule that rewrites the scalar between replays.  params / momentum_bufs: fp32; grads: fp32, or bf16 when
+ * grads_are_bf16 (the buckets of a bf16 all-reduce, read only: write_grads must be 0); shadows: bf16 or NULL (whole
+ * array or per tensor); momentum_bufs may be NULL when momentum == 0.  All tables are HOST arrays over the group's
+ * tensors (contiguous); norms_ws: device [2 * n_tensors] fp64 scratch (only when `lars`).  Two launches (norms,
+ * update) per 48 tensors. */
+int stswin_lars_sgd_step(void* const* params, void* const* grads, void* const* momentum_bufs, void* const* shadows,
+                         const int64_t* numels, const uint8_t* first_step, int n_tensors, int grads_are_bf16,
+                         int write_grads, float lr, const float* lr_dev, float momentum, float dampening, int nesterov,
+                         float weight_decay, int lars, float trust_coef, float eps, double* norms_ws, void* stream);
 
 /* Adam step over a list of tensors (the optimiser of seg18/train_swin.py: torch.optim.Adam, no amsgrad), emitting the
  * bf16 copy of the updated weights that the Swin kernels consume (replaces the optimiser's own pass plus one cast

@@ -94,9 +94,9 @@ SIGNATURES = {
     "stswin_ohem_ws_bytes": ([], ctypes.c_int64),
     "stswin_ohem_ce_fwd": ([_vp, _i, _vp, _i, _i, _i64, _i, ctypes.c_float, _i64, _fp, _vp, _fp, _fp, _vp], ctypes.c_int),
     "stswin_ohem_ce_bwd": ([_vp, _i, _vp, _i, _i, _i64, _i, _fp, _fp, _fp, _vp, _vp], ctypes.c_int),
-    "stswin_ema_update": ([_vp, _vp, _vp, _i, ctypes.c_float, ctypes.c_float, _vp], ctypes.c_int),
-    "stswin_lars_sgd_step": ([_vp, _vp, _vp, _vp, _vp, _i] + [ctypes.c_float] * 3 + [_i, ctypes.c_float, _i,
-                             ctypes.c_float, ctypes.c_float, _vp, _vp], ctypes.c_int),
+    "stswin_ema_update": ([_vp, _vp, _vp, _vp, _i, ctypes.c_float, ctypes.c_float, _fp, _vp], ctypes.c_int),
+    "stswin_lars_sgd_step": ([_vp] * 6 + [_i, _i, _i, ctypes.c_float, _fp] + [ctypes.c_float] * 2 + [_i, ctypes.c_float, _i,
+                             ctypes.c_float, ctypes.c_float, _fp, _vp], ctypes.c_int),
     "stswin_adam_step": ([_vp] * 6 + [_i, _i] + [ctypes.c_float] * 6 + [_vp, _vp], ctypes.c_int),
     "stswin_sgd_step": ([_vp] * 6 + [_i, _i, ctypes.c_float, _fp] + [ctypes.c_float] * 2 + [_i, _i] + [ctypes.c_float] * 2
                         + [_vp], ctypes.c_int),

@@ -5,7 +5,7 @@
 
 extern "C" {
 
-int stswin_abi_version(void) { return 5; }
+int stswin_abi_version(void) { return 6; }
 const char* stswin_last_error(void) { return stswin::last_error(); }
 int stswin_set_device(int device) {
   STSWIN_CUDA(cudaSetDevice(device));
@@ -99,16 +99,18 @@ int stswin_ohem_ce_bwd(const void* logits, int logits_is_f32, const int64_t* lab
   return stswin::ohem_ce_bwd(logits, logits_is_f32, labels, B, K, HW, ignore_index, loss_px, sel, d_loss, d_logits,
                              static_cast<cudaStream_t>(stream));
 }
-int stswin_ema_update(void* const* k_params, const void* const* q_params, const int64_t* numels, int n_tensors, float m,
-                      float one_minus_m, void* stream) {
-  return stswin::ema_update(k_params, q_params, numels, n_tensors, m, one_minus_m, static_cast<cudaStream_t>(stream));
+int stswin_ema_update(void* const* k_params, const void* const* q_params, void* const* k_shadows, const int64_t* numels,
+                      int n_tensors, float m, float one_minus_m, const float* m_dev, void* stream) {
+  return stswin::ema_update(k_params, q_params, k_shadows, numels, n_tensors, m, one_minus_m, m_dev,
+                            static_cast<cudaStream_t>(stream));
 }
-int stswin_lars_sgd_step(void* const* params, void* const* grads, void* const* momentum_bufs, const int64_t* numels,
-                         const uint8_t* first_step, int n_tensors, float lr, float momentum, float dampening,
-                         int nesterov, float weight_decay, int lars, float trust_coef, float eps, double* norms_ws,
-                         void* stream) {
-  return stswin::lars_sgd_step(params, grads, momentum_bufs, numels, first_step, n_tensors, lr, momentum, dampening,
-                               nesterov, weight_decay, lars, trust_coef, eps, norms_ws, static_cast<cudaStream_t>(stream));
+int stswin_lars_sgd_step(void* const* params, void* const* grads, void* const* momentum_bufs, void* const* shadows,
+                         const int64_t* numels, const uint8_t* first_step, int n_tensors, int grads_are_bf16,
+                         int write_grads, float lr, const float* lr_dev, float momentum, float dampening, int nesterov,
+                         float weight_decay, int lars, float trust_coef, float eps, double* norms_ws, void* stream) {
+  return stswin::lars_sgd_step(params, grads, momentum_bufs, shadows, numels, first_step, n_tensors, grads_are_bf16,
+                               write_grads, lr, lr_dev, momentum, dampening, nesterov, weight_decay, lars, trust_coef, eps,
+                               norms_ws, static_cast<cudaStream_t>(stream));
 }
 
 int stswin_adam_step(void* const* params, const void* const* grads, void* const* exp_avg, void* const* exp_avg_sq,

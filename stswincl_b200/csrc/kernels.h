@@ -46,11 +46,12 @@ int ohem_ce_fwd(const void* logits, int logits_is_f32, const int64_t* labels, in
                 float thresh, long n_min, float* loss_px, void* ws, float* loss, float* sel, cudaStream_t stream);
 int ohem_ce_bwd(const void* logits, int logits_is_f32, const int64_t* labels, int B, int K, long HW, int ignore_index,
                 const float* loss_px, const float* sel, const float* d_loss, void* d_logits, cudaStream_t stream);
-int ema_update(void* const* k_params, const void* const* q_params, const int64_t* numels, int n_tensors, float m,
-               float one_minus_m, cudaStream_t stream);
-int lars_sgd_step(void* const* params, void* const* grads, void* const* bufs, const int64_t* numels,
-                  const uint8_t* first_step, int n_tensors, float lr, float momentum, float dampening, int nesterov,
-                  float weight_decay, int lars, float trust_coef, float eps, double* norms_ws, cudaStream_t stream);
+int ema_update(void* const* k_params, const void* const* q_params, void* const* k_shadows, const int64_t* numels,
+               int n_tensors, float m, float one_minus_m, const float* m_dev, cudaStream_t stream);
+int lars_sgd_step(void* const* params, void* const* grads, void* const* bufs, void* const* shadows, const int64_t* numels,
+                  const uint8_t* first_step, int n_tensors, int grads_are_bf16, int write_grads, float lr,
+                  const float* lr_dev, float momentum, float dampening, int nesterov, float weight_decay, int lars,
+                  float trust_coef, float eps, double* norms_ws, cudaStream_t stream);
 
 int adam_step(void* const* params, const void* const* grads, void* const* exp_avg, void* const* exp_avg_sq,
               void* const* shadows, const int64_t* numels, int n_tensors, int grads_are_bf16, float lr, float beta1,

@@ -1,7 +1,8 @@
 // Training-step kernels either side of the two hot paths (SURVEY.md section 8f, rows N2-N4):
 //   * OHEM cross-entropy        -- OhemCELoss2D, seg18/utils/losses.py:16-40
-//   * key-encoder momentum (EMA) update -- PixPro._momentum_update_key_encoder, PixPro_swin_v5.py:258-289
-//   * LARS-scaled SGD step      -- contrast/lars.py:109-152 (+ torch.optim.SGD it wraps)
+//   * key-encoder momentum (EMA) update + bf16 key-weight shadow -- PixPro._momentum_update_key_encoder,
+//     PixPro_swin_v5.py:258-289
+//   * LARS-scaled SGD step + bf16 weight shadow -- contrast/lars.py:109-152 (+ torch.optim.SGD it wraps)
 //   * Adam step + bf16 weight shadow -- torch.optim.Adam of seg18/train_swin.py
 // All three are HBM-bound element streams: 16-byte accesses, grids sized from the SM count or the
 // element count, no host synchronisation (every data-dependent decision is taken on the device).
@@ -391,16 +392,39 @@ __device__ __forceinline__ int mt_find(const Args& t, int block) {
   return lo;
 }
 
-// param_k = param_k * m + param_q * (1 - m), rounded like the three eager ops of PixPro_swin_v5.py:266-267
-__global__ void __launch_bounds__(kThreads) ema_kernel(const __grid_constant__ MtArgs t, float m, float om) {
-  const int ti = mt_find(t, blockIdx.x);
-  float* __restrict__ k = static_cast<float*>(t.a[ti]);
-  const float* __restrict__ q = static_cast<const float*>(t.b[ti]);
-  const long n = t.numel[ti];
-  const long base = (long)(blockIdx.x - t.block_start[ti]) * MT_CHUNK;
+// MtArgs plus the bf16 shadow of each tensor `a` (null: none), for the streams that update a weight (EMA, LARS)
+struct ShArgs {
+  MtArgs m;
+  __nv_bfloat16* shadow[MT_MAX];
+};
+
+// gradients: fp32 (p.grad) or bf16 (the buckets of a bf16 all-reduce, widened exactly)
+__device__ __forceinline__ float4 load4(const float* g) { return *reinterpret_cast<const float4*>(g); }
+__device__ __forceinline__ float4 load4(const __nv_bfloat16* g) {
+  const uint2 raw = *reinterpret_cast<const uint2*>(g);
+  const float2 a = unpack_bf16(raw.x), b = unpack_bf16(raw.y);
+  return make_float4(a.x, a.y, b.x, b.y);
+}
+__device__ __forceinline__ float load1(const float* g) { return *g; }
+__device__ __forceinline__ float load1(const __nv_bfloat16* g) { return __bfloat162float(*g); }
+template <typename G>
+constexpr uintptr_t vec_align_mask() { return sizeof(G) == 4 ? 15 : 7; }
+
+// param_k = param_k * m + param_q * (1 - m), rounded like the three eager ops of PixPro_swin_v5.py:266-267; (m, 1 - m)
+// from m_dev[0..1] when m_dev is non-null (a schedule under graph replay); shadow = bf16_rn(param_k).  8 blocks per SM:
+// without the bound the shadow store takes the kernel to 38 registers and 6 blocks.
+__global__ void __launch_bounds__(kThreads, 8) ema_kernel(const __grid_constant__ ShArgs t, float m, float om,
+                                                       const float* __restrict__ m_dev) {
+  if (m_dev != nullptr) { m = __ldg(m_dev); om = __ldg(m_dev + 1); }
+  const int ti = mt_find(t.m, blockIdx.x);
+  float* __restrict__ k = static_cast<float*>(t.m.a[ti]);
+  const float* __restrict__ q = static_cast<const float*>(t.m.b[ti]);
+  __nv_bfloat16* __restrict__ sh = t.shadow[ti];
+  const long n = t.m.numel[ti];
+  const long base = (long)(blockIdx.x - t.m.block_start[ti]) * MT_CHUNK;
   const long end = base + MT_CHUNK < n ? base + MT_CHUNK : n;
   long i = base;
-  if ((((uintptr_t)k | (uintptr_t)q) & 15) == 0) {
+  if ((((uintptr_t)k | (uintptr_t)q) & 15) == 0 && (((uintptr_t)sh) & 7) == 0) {
     constexpr int U = 4;                                   // 8 independent 16-byte loads in flight per thread
     for (; i + U * kThreads * 4 <= end; i += U * kThreads * 4) {
       float4 kv[U], qv[U];
@@ -412,45 +436,56 @@ __global__ void __launch_bounds__(kThreads) ema_kernel(const __grid_constant__ M
       }
 #pragma unroll
       for (int u = 0; u < U; ++u) {
+        const long j = i + (long)(u * kThreads + threadIdx.x) * 4;
         kv[u].x = __fadd_rn(__fmul_rn(kv[u].x, m), __fmul_rn(qv[u].x, om));
         kv[u].y = __fadd_rn(__fmul_rn(kv[u].y, m), __fmul_rn(qv[u].y, om));
         kv[u].z = __fadd_rn(__fmul_rn(kv[u].z, m), __fmul_rn(qv[u].z, om));
         kv[u].w = __fadd_rn(__fmul_rn(kv[u].w, m), __fmul_rn(qv[u].w, om));
-        *reinterpret_cast<float4*>(k + i + (long)(u * kThreads + threadIdx.x) * 4) = kv[u];
+        *reinterpret_cast<float4*>(k + j) = kv[u];
+        if (sh != nullptr) *reinterpret_cast<uint2*>(sh + j) = make_uint2(pack_bf16(kv[u].x, kv[u].y), pack_bf16(kv[u].z, kv[u].w));
       }
     }
   }
-  for (long j = i + threadIdx.x; j < end; j += kThreads) k[j] = __fadd_rn(__fmul_rn(k[j], m), __fmul_rn(q[j], om));
+  for (long j = i + threadIdx.x; j < end; j += kThreads) {
+    const float v = __fadd_rn(__fmul_rn(k[j], m), __fmul_rn(q[j], om));
+    k[j] = v;
+    if (sh != nullptr) sh[j] = __float2bfloat16_rn(v);
+  }
 }
 
-// sum p^2 and sum (g + wd p)^2 per tensor (lars.py:121-127), fp64 accumulators norms[2*t], norms[2*t+1]
-__global__ void __launch_bounds__(kThreads) lars_norm_kernel(const __grid_constant__ MtArgs t, float wd, double* __restrict__ norms) {
-  const int ti = mt_find(t, blockIdx.x);
-  const float* __restrict__ p = static_cast<const float*>(t.a[ti]);
-  const float* __restrict__ g = static_cast<const float*>(t.b[ti]);
-  const long n = t.numel[ti];
-  const long base = (long)(blockIdx.x - t.block_start[ti]) * MT_CHUNK;
+// sum p^2 and sum (g + wd p)^2 per tensor (lars.py:121-127), fp64 accumulators norms[2*t], norms[2*t+1].  Every
+// rounding is spelled out (the contraction the fp32-only kernel had from nvcc), so it does not depend on the
+// gradient type or on the compiler's choices.
+__device__ __forceinline__ float sumsq4(float a, float b, float c, float d) {
+  return __fmaf_rn(d, d, __fmaf_rn(c, c, __fmaf_rn(a, a, __fmul_rn(b, b))));
+}
+
+template <typename G>
+__global__ void __launch_bounds__(kThreads) lars_norm_kernel(const __grid_constant__ ShArgs t, float wd, double* __restrict__ norms) {
+  const int ti = mt_find(t.m, blockIdx.x);
+  const float* __restrict__ p = static_cast<const float*>(t.m.a[ti]);
+  const G* __restrict__ g = static_cast<const G*>(t.m.b[ti]);
+  const long n = t.m.numel[ti];
+  const long base = (long)(blockIdx.x - t.m.block_start[ti]) * MT_CHUNK;
   const long end = base + MT_CHUNK < n ? base + MT_CHUNK : n;
   float sp = 0.f, sg = 0.f;
-  if ((((uintptr_t)p | (uintptr_t)g) & 15) == 0) {
+  long i = base + threadIdx.x;
+  if (((uintptr_t)p & 15) == 0 && ((uintptr_t)g & vec_align_mask<G>()) == 0) {
     const long end4 = base + ((end - base) & ~3L);
 #pragma unroll 4
-    for (long i = base + threadIdx.x * 4; i < end4; i += kThreads * 4) {
+    for (i = base + threadIdx.x * 4; i < end4; i += kThreads * 4) {
       const float4 pv = __ldg(reinterpret_cast<const float4*>(p + i));
-      const float4 gv = __ldg(reinterpret_cast<const float4*>(g + i));
-      const float g0 = gv.x + wd * pv.x, g1 = gv.y + wd * pv.y, g2 = gv.z + wd * pv.z, g3 = gv.w + wd * pv.w;
-      sp += pv.x * pv.x + pv.y * pv.y + pv.z * pv.z + pv.w * pv.w;
-      sg += g0 * g0 + g1 * g1 + g2 * g2 + g3 * g3;
+      const float4 gv = load4(g + i);
+      const float g0 = __fmaf_rn(wd, pv.x, gv.x), g1 = __fmaf_rn(wd, pv.y, gv.y), g2 = __fmaf_rn(wd, pv.z, gv.z),
+                  g3 = __fmaf_rn(wd, pv.w, gv.w);
+      sp = __fadd_rn(sumsq4(pv.x, pv.y, pv.z, pv.w), sp);
+      sg = __fadd_rn(sumsq4(g0, g1, g2, g3), sg);
     }
-    for (long i = end4 + threadIdx.x; i < end; i += kThreads) {
-      const float gg = g[i] + wd * p[i];
-      sp += p[i] * p[i]; sg += gg * gg;
-    }
-  } else {
-    for (long i = base + threadIdx.x; i < end; i += kThreads) {
-      const float gg = g[i] + wd * p[i];
-      sp += p[i] * p[i]; sg += gg * gg;
-    }
+    i = end4 + threadIdx.x;
+  }
+  for (; i < end; i += kThreads) {
+    const float pv = p[i], gg = __fmaf_rn(wd, pv, load1(g + i));
+    sp = __fmaf_rn(pv, pv, sp); sg = __fmaf_rn(gg, gg, sg);
   }
   __shared__ float s_p[kThreads / 32], s_g[kThreads / 32];
   sp = warp_sum(sp); sg = warp_sum(sg);
@@ -467,65 +502,86 @@ __global__ void __launch_bounds__(kThreads) lars_norm_kernel(const __grid_consta
 struct SgdArgs {
   float lr, momentum, dampening, wd, trust, eps;
   int nesterov, lars;
+  int store_grad;                    // fp32 gradients only: grad <- the decayed / scaled gradient (the p.grad contract)
+  const float* lr_dev;               // device scalar read instead of lr when non-null (a schedule under graph replay)
 };
 
-// g = grad + wd p; g *= trust |p| / (|g| + eps) (LARS group); grad = g; buf = momentum buf + (1 - dampening) g
-// (buf = g on a tensor's first step); p -= lr * buf        (lars.py:109-135 then torch.optim.SGD with wd 0, :137-152)
-__global__ void __launch_bounds__(kThreads) lars_sgd_kernel(const __grid_constant__ MtArgs t, const SgdArgs a,
+// g = grad + wd p; g *= trust |p| / (|g| + eps) (LARS group); grad = g (store_grad); buf = momentum buf + (1 - dampening) g
+// (buf = g on a tensor's first step); p -= lr * buf; shadow = bf16_rn(p)
+// (lars.py:109-135 then torch.optim.SGD with wd 0, :137-152).  Each rounding is spelled out as nvcc contracted the
+// fp32-only kernel: fma(wd, p, grad), one product by the LARS factor, fma(momentum, buf, g) for nesterov,
+// fma(-lr, d, p), and the momentum update as fma(1 - dampening, g, momentum * buf) on the 16-byte path but
+// fma(momentum, buf, (1 - dampening) * g) on the scalar tails and the unaligned path, so that every element keeps
+// the value that kernel gave it.
+template <typename G>
+__global__ void __launch_bounds__(kThreads) lars_sgd_kernel(const __grid_constant__ ShArgs t, const SgdArgs a,
                                                             const double* __restrict__ norms) {
-  const int ti = mt_find(t, blockIdx.x);
-  float* __restrict__ p = static_cast<float*>(t.a[ti]);
-  float* __restrict__ g = static_cast<float*>(t.b[ti]);
-  float* __restrict__ buf = static_cast<float*>(t.c[ti]);
-  const bool first = t.flag[ti] != 0;
-  const long n = t.numel[ti];
-  const long base = (long)(blockIdx.x - t.block_start[ti]) * MT_CHUNK;
+  const int ti = mt_find(t.m, blockIdx.x);
+  float* __restrict__ p = static_cast<float*>(t.m.a[ti]);
+  G* __restrict__ g = static_cast<G*>(t.m.b[ti]);
+  float* __restrict__ buf = static_cast<float*>(t.m.c[ti]);
+  __nv_bfloat16* __restrict__ sh = t.shadow[ti];
+  const bool first = t.m.flag[ti] != 0;
+  const long n = t.m.numel[ti];
+  const long base = (long)(blockIdx.x - t.m.block_start[ti]) * MT_CHUNK;
   const long end = base + MT_CHUNK < n ? base + MT_CHUNK : n;
+  const float neg_lr = -(a.lr_dev != nullptr ? __ldg(a.lr_dev) : a.lr);
+  const float one_minus_damp = __fsub_rn(1.f, a.dampening);
   float alr = 1.f;
   if (a.lars) {
     const float pn = (float)sqrt(norms[2 * ti]), gn = (float)sqrt(norms[2 * ti + 1]);
-    if (pn > 0.f && gn > 0.f) alr = a.trust * pn / (gn + a.eps);
+    if (pn > 0.f && gn > 0.f) alr = __fdiv_rn(__fmul_rn(a.trust, pn), __fadd_rn(gn, a.eps));
   }
-  auto one = [&](float pv, float gv, float bv, float& p_out, float& g_out, float& b_out) {
-    float gg = a.wd > 0.f ? gv + a.wd * pv : gv;
-    if (a.lars) gg *= alr;
+  const bool has_buf = a.momentum != 0.f;
+  constexpr bool kF32 = sizeof(G) == 4;
+  const bool store_grad = kF32 && a.store_grad;
+  auto one = [&](float pv, float gv, float& bv, float& g_out, bool vec) -> float {
+    float gg = a.wd > 0.f ? __fmaf_rn(a.wd, pv, gv) : gv;
+    if (a.lars) gg = __fmul_rn(gg, alr);
     g_out = gg;
     float d = gg;
-    if (a.momentum != 0.f) {
-      b_out = first ? gg : a.momentum * bv + (1.f - a.dampening) * gg;
-      d = a.nesterov ? gg + a.momentum * b_out : b_out;
+    if (has_buf) {
+      bv = first ? gg
+           : vec ? __fmaf_rn(one_minus_damp, gg, __fmul_rn(a.momentum, bv))
+                 : __fmaf_rn(a.momentum, bv, __fmul_rn(one_minus_damp, gg));
+      d = a.nesterov ? __fmaf_rn(a.momentum, bv, gg) : bv;
     }
-    p_out = pv - a.lr * d;
+    return __fmaf_rn(neg_lr, d, pv);
   };
-  const bool has_buf = a.momentum != 0.f;
-  if ((((uintptr_t)p | (uintptr_t)g | (uintptr_t)buf) & 15) == 0) {
+  long i = base + threadIdx.x;
+  if ((((uintptr_t)p | (uintptr_t)buf) & 15) == 0 && ((uintptr_t)g & vec_align_mask<G>()) == 0 && ((uintptr_t)sh & 7) == 0) {
     const long end4 = base + ((end - base) & ~3L);
 #pragma unroll 2
-    for (long i = base + threadIdx.x * 4; i < end4; i += kThreads * 4) {
+    for (i = base + threadIdx.x * 4; i < end4; i += kThreads * 4) {
       float4 pv = *reinterpret_cast<const float4*>(p + i);
-      float4 gv = *reinterpret_cast<const float4*>(g + i);
+      float4 gv = load4(g + i);
       float4 bv = (has_buf && !first) ? *reinterpret_cast<const float4*>(buf + i) : make_float4(0.f, 0.f, 0.f, 0.f);
-      one(pv.x, gv.x, bv.x, pv.x, gv.x, bv.x);
-      one(pv.y, gv.y, bv.y, pv.y, gv.y, bv.y);
-      one(pv.z, gv.z, bv.z, pv.z, gv.z, bv.z);
-      one(pv.w, gv.w, bv.w, pv.w, gv.w, bv.w);
+      pv.x = one(pv.x, gv.x, bv.x, gv.x, true);
+      pv.y = one(pv.y, gv.y, bv.y, gv.y, true);
+      pv.z = one(pv.z, gv.z, bv.z, gv.z, true);
+      pv.w = one(pv.w, gv.w, bv.w, gv.w, true);
       *reinterpret_cast<float4*>(p + i) = pv;
-      *reinterpret_cast<float4*>(g + i) = gv;
+      if constexpr (kF32) {
+        if (store_grad) *reinterpret_cast<float4*>(g + i) = gv;
+      }
       if (has_buf) *reinterpret_cast<float4*>(buf + i) = bv;
+      if (sh != nullptr) *reinterpret_cast<uint2*>(sh + i) = make_uint2(pack_bf16(pv.x, pv.y), pack_bf16(pv.z, pv.w));
     }
-    for (long i = end4 + threadIdx.x; i < end; i += kThreads) {
-      float bv = (has_buf && !first) ? buf[i] : 0.f;
-      one(p[i], g[i], bv, p[i], g[i], bv);
-      if (has_buf) buf[i] = bv;
+    i = end4 + threadIdx.x;
+  }
+  for (; i < end; i += kThreads) {
+    float bv = (has_buf && !first) ? buf[i] : 0.f, gv;
+    const float pv = one(p[i], load1(g + i), bv, gv, false);
+    p[i] = pv;
+    if constexpr (kF32) {
+      if (store_grad) g[i] = gv;
     }
-  } else {
-    for (long i = base + threadIdx.x; i < end; i += kThreads) {
-      float bv = (has_buf && !first) ? buf[i] : 0.f;
-      one(p[i], g[i], bv, p[i], g[i], bv);
-      if (has_buf) buf[i] = bv;
-    }
+    if (has_buf) buf[i] = bv;
+    if (sh != nullptr) sh[i] = __float2bfloat16_rn(pv);
   }
 }
+// the whole argument block of the largest of these launches stays within the 4 KB kernel-parameter limit
+static_assert(sizeof(ShArgs) + sizeof(SgdArgs) + sizeof(double*) <= 4096, "lars_sgd_kernel parameters exceed 4 KB");
 
 // ------------------------------------------------------------------------------------------------
 // Adam (torch.optim.Adam semantics, no amsgrad) as a multi-tensor stream that also emits the bf16 shadow of the
@@ -798,37 +854,52 @@ int ohem_ce_bwd(const void* logits, int logits_is_f32, const int64_t* labels, in
   return kOk;
 }
 
-int ema_update(void* const* k_params, const void* const* q_params, const int64_t* numels, int n_tensors, float m,
-               float one_minus_m, cudaStream_t stream) {
+// fill ShArgs for tensors [t0, t0 + cnt); returns the number of blocks
+int sh_fill(ShArgs& s, void* const* a, const void* const* b, void* const* c, void* const* shadows, const int64_t* numels,
+            const uint8_t* flags, int t0, int cnt) {
+  for (int i = 0; i < cnt; ++i) s.shadow[i] = shadows ? static_cast<__nv_bfloat16*>(shadows[t0 + i]) : nullptr;
+  return mt_fill(s.m, a, const_cast<void* const*>(b), c, numels, flags, t0, cnt);
+}
+
+int ema_update(void* const* k_params, const void* const* q_params, void* const* k_shadows, const int64_t* numels,
+               int n_tensors, float m, float one_minus_m, const float* m_dev, cudaStream_t stream) {
   STSWIN_CHECK_ARG(n_tensors >= 0 && (n_tensors == 0 || (k_params && q_params && numels)), "ema_update: null table");
   for (int t0 = 0; t0 < n_tensors; t0 += MT_MAX) {
-    MtArgs args;
+    ShArgs args;
     const int cnt = n_tensors - t0 < MT_MAX ? n_tensors - t0 : MT_MAX;
-    const int blocks = mt_fill(args, k_params, const_cast<void* const*>(q_params), nullptr, numels, nullptr, t0, cnt);
+    const int blocks = sh_fill(args, k_params, q_params, nullptr, k_shadows, numels, nullptr, t0, cnt);
     if (blocks == 0) continue;
-    ema_kernel<<<blocks, kThreads, 0, stream>>>(args, m, one_minus_m);
+    ema_kernel<<<blocks, kThreads, 0, stream>>>(args, m, one_minus_m, m_dev);
   }
   STSWIN_CUDA(cudaGetLastError());
   return kOk;
 }
 
-int lars_sgd_step(void* const* params, void* const* grads, void* const* bufs, const int64_t* numels,
-                  const uint8_t* first_step, int n_tensors, float lr, float momentum, float dampening, int nesterov,
-                  float weight_decay, int lars, float trust_coef, float eps, double* norms_ws, cudaStream_t stream) {
+int lars_sgd_step(void* const* params, void* const* grads, void* const* bufs, void* const* shadows, const int64_t* numels,
+                  const uint8_t* first_step, int n_tensors, int grads_are_bf16, int write_grads, float lr,
+                  const float* lr_dev, float momentum, float dampening, int nesterov, float weight_decay, int lars,
+                  float trust_coef, float eps, double* norms_ws, cudaStream_t stream) {
   STSWIN_CHECK_ARG(n_tensors >= 0 && (n_tensors == 0 || (params && grads && numels)), "lars_sgd_step: null table");
   STSWIN_CHECK_ARG(momentum == 0.f || bufs != nullptr, "lars_sgd_step: momentum needs momentum buffers");
   STSWIN_CHECK_ARG(!lars || norms_ws != nullptr, "lars_sgd_step: the LARS group needs a [2*n_tensors] fp64 workspace");
   STSWIN_CHECK_ARG(!nesterov || (momentum > 0.f && dampening == 0.f), "lars_sgd_step: nesterov needs momentum and zero dampening");
+  STSWIN_CHECK_ARG(!(grads_are_bf16 && write_grads), "lars_sgd_step: bf16 gradients are read-only (write_grads needs fp32)");
   if (n_tensors == 0) return kOk;
   if (lars) STSWIN_CUDA(cudaMemsetAsync(norms_ws, 0, sizeof(double) * 2 * (size_t)n_tensors, stream));
-  const SgdArgs a{lr, momentum, dampening, weight_decay, trust_coef, eps, nesterov, lars};
+  const SgdArgs a{lr, momentum, dampening, weight_decay, trust_coef, eps, nesterov, lars, write_grads, lr_dev};
   for (int t0 = 0; t0 < n_tensors; t0 += MT_MAX) {
-    MtArgs args;
+    ShArgs args;
     const int cnt = n_tensors - t0 < MT_MAX ? n_tensors - t0 : MT_MAX;
-    const int blocks = mt_fill(args, params, grads, momentum != 0.f ? bufs : nullptr, numels, first_step, t0, cnt);
+    const int blocks = sh_fill(args, params, grads, momentum != 0.f ? bufs : nullptr, shadows, numels, first_step, t0, cnt);
     if (blocks == 0) continue;
-    if (lars) lars_norm_kernel<<<blocks, kThreads, 0, stream>>>(args, weight_decay, norms_ws + 2 * t0);
-    lars_sgd_kernel<<<blocks, kThreads, 0, stream>>>(args, a, norms_ws ? norms_ws + 2 * t0 : nullptr);
+    double* nw = norms_ws ? norms_ws + 2 * t0 : nullptr;
+    if (grads_are_bf16) {
+      if (lars) lars_norm_kernel<__nv_bfloat16><<<blocks, kThreads, 0, stream>>>(args, weight_decay, nw);
+      lars_sgd_kernel<__nv_bfloat16><<<blocks, kThreads, 0, stream>>>(args, a, nw);
+    } else {
+      if (lars) lars_norm_kernel<float><<<blocks, kThreads, 0, stream>>>(args, weight_decay, nw);
+      lars_sgd_kernel<float><<<blocks, kThreads, 0, stream>>>(args, a, nw);
+    }
   }
   STSWIN_CUDA(cudaGetLastError());
   return kOk;

@@ -126,7 +126,7 @@ class SegmentedStep:
     optimizer step are issued between / after the replays.
 
     The optimizer step reads the reduced gradients straight from the buckets when the optimizer accepts
-    ``step(grads=...)`` (``optim.FusedAdam``, ``optim.FusedSGD``: fp32 or bf16 gradients); otherwise they are copied back into
+    ``step(grads=...)`` (``optim.FusedAdam``, ``optim.FusedSGD``, ``optim.LARS``: fp32 or bf16 gradients); otherwise they are copied back into
     ``p.grad`` first.  Backend-agnostic (NCCL on GPUs, gloo in the CPU tests; there ``use_graph=False``)."""
 
     def __init__(self, model, optimizer, loss_fn, *, segments: int = 4, wire_dtype: torch.dtype = torch.bfloat16,

@@ -12,9 +12,11 @@
     synchronisation for every weight tensor and step; here each parameter group is two multi-tensor
     launches (norms, update) per 48 tensors with every decision taken on the device
     (``stswin_lars_sgd_step``).  State stays in the wrapped optimiser (``momentum_buffer``), so
-    ``state_dict`` / ``load_state_dict`` interoperate with the reference.
+    ``state_dict`` / ``load_state_dict`` interoperate with the reference.  The same contract as ``FusedSGD``: the
+    bf16 weight shadow, ``step(grads=...)`` over fp32 or bf16 bucket gradients, and a device-tensor ``lr``.
   * ``momentum_update``              -- the key-encoder EMA of ``PixPro._momentum_update_key_encoder``
-    (``PixPro_swin_v5.py:258-289``): one multi-tensor stream instead of three eager ops per parameter.
+    (``PixPro_swin_v5.py:258-289``): one multi-tensor stream instead of three eager ops per parameter, writing the
+    bf16 shadow of the key weights; the momentum may be a device pair, so a captured update follows a schedule.
 
 CUDA fp32 parameters only -- no CPU path.
 """
@@ -60,11 +62,18 @@ def _numels(tensors: Sequence[torch.Tensor]):
 
 
 @torch.no_grad()
-def momentum_update(params_q: Iterable[torch.Tensor], params_k: Iterable[torch.Tensor], momentum: float) -> None:
+def momentum_update(params_q: Iterable[torch.Tensor], params_k: Iterable[torch.Tensor], momentum, *,
+                    shadow: bool = True) -> None:
     """``param_k = param_k * momentum + param_q * (1. - momentum)`` for every pair, in place
-    (``PixPro_swin_v5.py:266-267``), bit-exact with the eager expression."""
+    (``PixPro_swin_v5.py:266-267``), bit-exact with the eager expression.
+
+    ``momentum`` is a float, or a 2-element fp32 tensor ``[m, 1 - m]`` on the parameters' device, read by the kernel
+    on the device (a CUDA-graph-captured update then follows a schedule written into the tensor between replays); for
+    bit-exactness its entries are the fp32 roundings of the double ``m`` and ``1. - m``.  With ``shadow``, every key
+    parameter of >= 2 dimensions keeps a bf16 shadow that the update rewrites (``bf16_weight``)."""
+    pk = list(params_k)
     q = [p.data for p in params_q]
-    k = [p.data for p in params_k]
+    k = [p.data for p in pk]
     if len(q) != len(k):
         raise ValueError(f"momentum_update: {len(q)} query tensors vs {len(k)} key tensors")
     if not q:
@@ -73,17 +82,47 @@ def momentum_update(params_q: Iterable[torch.Tensor], params_k: Iterable[torch.T
     for a, b in zip(q, k):
         if a.shape != b.shape or a.device != b.device:
             raise ValueError("momentum_update: query / key parameter mismatch")
-    n_bytes = sum(t.numel() for t in k) * 4
-    with ops._launch("ema_update", 3.0 * n_bytes, k[0]):                     # read k, q; write k
-        st = _lib.load().stswin_ema_update(_ptrs(k), _ptrs(q), _numels(k), len(k), float(momentum), float(1. - momentum),
-                                           ops._stream(k[0]))
+    if torch.is_tensor(momentum):
+        if momentum.dtype != torch.float32 or momentum.shape != (2,) or momentum.device != k[0].device or \
+                not momentum.is_contiguous():
+            raise StswinError(f"momentum_update: a tensor momentum must be the contiguous fp32 pair [m, 1 - m] on "
+                              f"{k[0].device}, got {momentum.dtype} {tuple(momentum.shape)} on {momentum.device}")
+        m, om, m_dev = 0.0, 0.0, momentum.data_ptr()
+    else:
+        m, om, m_dev = float(momentum), float(1. - momentum), None
+    shadows = [_shadow_ptr(p, shadow) for p in pk]
+    n_bytes = sum(t.numel() for t in k) * 12 + sum(t.numel() for t, s in zip(k, shadows) if s is not None) * 2
+    with ops._launch("ema_update", float(n_bytes), k[0]):                   # read k, q; write k (+ shadow)
+        st = _lib.load().stswin_ema_update(_ptrs(k), _ptrs(q), (ctypes.c_void_p * len(shadows))(*shadows), _numels(k),
+                                           len(k), m, om, m_dev, ops._stream(k[0]))
     _lib.check(st, "stswin_ema_update")
 
 
-class LARS(Optimizer):
-    """'LARS (Layer-wise Adaptive Rate Scaling)' as a wrapper of ``torch.optim.SGD`` (``lars.py:34-152``)."""
+def _lr_arg(lr, dev, who: str):
+    """(host lr, device lr pointer) of a group's ``lr``: a number, or a 0-dim fp32 tensor on ``dev`` that the kernel
+    reads on the device."""
+    if not torch.is_tensor(lr):
+        return float(lr), None
+    if lr.dim() != 0 or lr.dtype != torch.float32 or lr.device != dev:
+        raise StswinError(f"{who}: a tensor lr must be a 0-dim fp32 tensor on {dev}, got {lr.dtype} "
+                          f"{tuple(lr.shape)} on {lr.device}")
+    return 0.0, lr.data_ptr()
 
-    def __init__(self, optimizer, eps=1e-8, trust_coef=0.001):
+
+class LARS(Optimizer):
+    """'LARS (Layer-wise Adaptive Rate Scaling)' as a wrapper of ``torch.optim.SGD`` (``lars.py:34-152``).
+
+    With ``shadow``, the update pass also writes the bf16 shadow of every >= 2-D parameter (``bf16_weight``).  A
+    group's ``lr`` may be a 0-dim fp32 CUDA tensor (``torch.optim.SGD(..., lr=lr_t)``): the kernel reads it on the
+    device, so a CUDA-graph-captured step follows a schedule that writes the tensor between replays.  The step is
+    capturable once every momentum buffer exists (after one eager step).
+
+    ``step(grads=...)`` takes the gradients from a list (fp32 or bf16, one per ``requires_grad`` parameter in group
+    order) instead of ``p.grad`` -- the bucket views of a data-parallel all-reduce (``dist.SegmentedStep``).  On that
+    path neither ``p.grad`` nor the list is written; on the ``p.grad`` path ``p.grad`` holds the decayed / scaled
+    gradient afterwards, as in the reference."""
+
+    def __init__(self, optimizer, eps=1e-8, trust_coef=0.001, *, shadow: bool = True):
         if eps < 0.0:
             raise ValueError('invalid epsilon value: , %f' % eps)
         if trust_coef < 0.0:
@@ -93,14 +132,16 @@ class LARS(Optimizer):
         self.optim = optimizer
         self.eps = eps
         self.trust_coef = trust_coef
+        self.shadow = shadow
 
     def __getstate__(self):
-        return (self.optim, {'eps': self.eps, 'trust_coef': self.trust_coef})
+        return (self.optim, {'eps': self.eps, 'trust_coef': self.trust_coef, 'shadow': self.shadow})
 
     def __setstate__(self, state):
         self.optim, lars_dict = state
         self.eps = lars_dict['eps']
         self.trust_coef = lars_dict['trust_coef']
+        self.shadow = lars_dict.get('shadow', True)
 
     def __repr__(self):
         return '%s(%r)' % (self.__class__.__name__, self.optim)
@@ -126,22 +167,38 @@ class LARS(Optimizer):
         self.optim.add_param_group(param_group)
 
     @torch.no_grad()
-    def step(self, closure=None):
+    def step(self, closure=None, grads=None):
         """Weight decay into the gradient, LARS scaling of the non-``ignore`` group, momentum SGD update
-        (``lars.py:109-152``); ``p.grad`` holds the decayed / scaled gradient afterwards, as in the reference."""
+        (``lars.py:109-152``), from ``p.grad`` or from ``grads`` (see the class docstring)."""
         loss = None
         if closure is not None:
             with torch.enable_grad():
                 loss = closure()
         lib = _lib.load()
+        if grads is not None:
+            n_req = sum(p.requires_grad for group in self.optim.param_groups for p in group['params'])
+            if len(grads) != n_req:
+                raise StswinError(f"LARS.step: {len(grads)} gradients for {n_req} parameters that require grad")
+        gi = 0
         for group in self.optim.param_groups:
-            params = [p for p in group['params'] if p.grad is not None]
+            if grads is None:
+                params = [p for p in group['params'] if p.grad is not None]
+                gl = [p.grad for p in params]
+            else:
+                params = [p for p in group['params'] if p.requires_grad]
+                gl = list(grads[gi:gi + len(params)])
+                gi += len(params)
             if not params:
                 continue
             if group.get('maximize', False):
                 raise StswinError("LARS: maximize=True is not supported")
-            grads = [p.grad for p in params]
-            _check_f32(params, "LARS.step"); _check_f32(grads, "LARS.step (grad)")
+            _check_f32(params, "LARS.step")
+            gdt = gl[0].dtype
+            if gdt not in (torch.float32, torch.bfloat16) or any(g.dtype != gdt or not g.is_contiguous() or not g.is_cuda or
+                                                                 g.numel() != p.numel() for g, p in zip(gl, params)):
+                raise StswinError("LARS.step: gradients must be contiguous CUDA tensors, all fp32 or all bf16, one per "
+                                  "parameter and of its size")
+            lr, lr_dev = _lr_arg(group['lr'], params[0].device, "LARS.step")
             momentum, dampening = float(group['momentum']), float(group['dampening'])
             ignore = group.get('ignore', None)
             lars = ignore is not None and not ignore          # lars.py:125
@@ -157,14 +214,20 @@ class LARS(Optimizer):
                     bufs.append(buf)
                 _check_f32(bufs, "LARS.step (momentum_buffer)")
                 first = (ctypes.c_uint8 * len(flags))(*flags)
+            shadows = [_shadow_ptr(p, self.shadow) for p in params]
             dev = params[0].device
             norms = torch.empty(2 * len(params), dtype=torch.float64, device=dev) if lars else None
-            n_bytes = sum(p.numel() for p in params) * 4
-            passes = (2 if lars else 0) + 4 + (2 if momentum != 0 else 0)       # norms: p, g; update: p, g in / out (+ buf)
-            with ops._launch("lars_sgd_step", float(passes * n_bytes), params[0]):
-                st = lib.stswin_lars_sgd_step(_ptrs(params), _ptrs(grads), _ptrs(bufs) if bufs else None, _numels(params), first,
-                                              len(params), float(group['lr']), momentum, dampening, int(bool(group['nesterov'])),
-                                              float(group['weight_decay']), int(lars), float(self.trust_coef), float(self.eps),
+            write = grads is None                                               # the p.grad contract of the reference
+            n_el, gsz = sum(p.numel() for p in params), gl[0].element_size()
+            # norms: p, g; update: p in / out, g in (+ out), buf in / out, shadow out
+            n_bytes = n_el * ((4 + gsz if lars else 0) + 8 + gsz + (4 if write else 0) + (8 if momentum != 0 else 0)) + \
+                sum(p.numel() for p, s in zip(params, shadows) if s is not None) * 2
+            with ops._launch("lars_sgd_step", float(n_bytes), params[0]):
+                st = lib.stswin_lars_sgd_step(_ptrs(params), _ptrs(gl), _ptrs(bufs) if bufs else None,
+                                              (ctypes.c_void_p * len(shadows))(*shadows), _numels(params), first,
+                                              len(params), int(gdt == torch.bfloat16), int(write), lr, lr_dev, momentum,
+                                              dampening, int(bool(group['nesterov'])), float(group['weight_decay']),
+                                              int(lars), float(self.trust_coef), float(self.eps),
                                               norms.data_ptr() if norms is not None else None, ops._stream(params[0]))
             _lib.check(st, "stswin_lars_sgd_step")
         return loss
@@ -174,8 +237,8 @@ class LARS(Optimizer):
 # bf16 shadow of the weights
 # ---------------------------------------------------------------------------------------------------------------
 def bf16_weight(w: torch.Tensor) -> torch.Tensor:
-    """The bf16 copy of a weight the GEMM kernels consume.  ``FusedAdam`` and ``FusedSGD`` keep a shadow copy per
-    parameter that their update kernel rewrites every step, so the forward needs no cast kernel; the shadow is valid as long as nobody else
+    """The bf16 copy of a weight the GEMM kernels consume.  ``FusedAdam``, ``FusedSGD``, ``LARS`` and
+    ``momentum_update`` (key weights) keep a shadow copy per parameter that their update kernel rewrites every step, so the forward needs no cast kernel; the shadow is valid as long as nobody else
     wrote the parameter (tracked by the tensor's version counter -- the kernel does not bump it).  Without a valid
     shadow this is ``w.to(bfloat16)``."""
     sh = getattr(w, "_stswin_shadow", None)
@@ -311,16 +374,6 @@ class FusedSGD(Optimizer):
             group.setdefault("nesterov", False)
             group.setdefault("maximize", False)
 
-    @staticmethod
-    def _lr(lr, dev):
-        """(host lr, device lr pointer) of a group's ``lr``."""
-        if not torch.is_tensor(lr):
-            return float(lr), None
-        if lr.dim() != 0 or lr.dtype != torch.float32 or lr.device != dev:
-            raise StswinError(f"FusedSGD.step: a tensor lr must be a 0-dim fp32 tensor on {dev}, got {lr.dtype} "
-                              f"{tuple(lr.shape)} on {lr.device}")
-        return 0.0, lr.data_ptr()
-
     @torch.no_grad()
     def step(self, closure=None, grads=None, grad_scale: float = 1.0):
         loss = None
@@ -347,7 +400,7 @@ class FusedSGD(Optimizer):
                                                                  g.numel() != p.numel() for g, p in zip(gl, params)):
                 raise StswinError("FusedSGD.step: gradients must be contiguous CUDA tensors, all fp32 or all bf16, one per "
                                   "parameter and of its size")
-            lr, lr_dev = self._lr(group["lr"], params[0].device)
+            lr, lr_dev = _lr_arg(group["lr"], params[0].device, "FusedSGD.step")
             momentum = float(group["momentum"])
             bufs, first = None, None
             if momentum != 0:

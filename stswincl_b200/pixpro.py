@@ -10,7 +10,8 @@ the part of that class that touches the two hot paths:
     ``swin`` in both by ``stswincl_b200.swin.SwinTransformerLayerv5`` (``encoder_2`` / ``encoder_k_2``, :166,181),
     loading the reference weights strictly;
   * ``_momentum_update_key_encoder`` (:258-289) is one multi-tensor EMA launch per 48 tensors over ALL parameter
-    pairs (``optim.momentum_update``), with the cosine momentum schedule of :262;
+    pairs (``optim.momentum_update``), with the cosine momentum schedule of :262 kept on the device (a table of the
+    per-iteration momenta and a device step counter), so a CUDA-graph-captured ``forward`` follows the schedule;
   * the 6 key passes run through the forward-only block path (no activations kept, no GELU-derivative output);
   * ``forward`` returns the reference's 8-tuple; with ``fuse_normalize=True`` the embeddings are returned
     un-normalised for ``contrast.consistency_loss_tail(normalize=True)``, which fuses ``F.normalize`` (:330,...).
@@ -41,6 +42,20 @@ def swap_swin_head(segmentor: nn.Module, attr: str = "swin") -> nn.Module:
     p = next(old.parameters())
     setattr(segmentor, attr, new.to(p.device))
     return segmentor
+
+
+def momentum_table(base_momentum: float, K: int) -> torch.Tensor:
+    """fp32 [K + 1, 2]: row k < K is (m_k, 1 - m_k) with m_k = 1 - (1 - base) (cos(pi k / K) + 1) / 2 evaluated in
+    double, as PixPro_swin_v5.py:262 does, and each entry rounded to fp32 once -- the values the eager expression
+    ``k * m + q * (1. - m)`` multiplies by.  Row K is (1, 0), the expression's own value at k = K; every k >= K reads
+    it, so past the end of the schedule the key encoder stays where it is (the expression would start a second cosine
+    period there, which no recipe reaches: K is the recipe's iteration count)."""
+    rows = []
+    for k in range(K):
+        m = 1. - (1. - base_momentum) * (math.cos(math.pi * k / K) + 1) / 2.
+        rows.append((m, 1. - m))
+    rows.append((1., 0.))
+    return torch.tensor(rows, dtype=torch.float32)
 
 
 class PixPro(nn.Module):
@@ -78,7 +93,25 @@ class PixPro(nn.Module):
             raise NotImplementedError("pixpro_transform_layer 2 (MLP2d) is the caller's module: assign value_transform")
         # momentum schedule length and position (:230-231)
         self.K = int(args.num_instances * 1. / world_size / args.batch_size * args.epochs)
+        if self.K < 1:
+            raise ValueError(f"PixPro: the momentum schedule needs at least one iteration, got K = {self.K}")
+        # the schedule on the device (momentum_table) and its position; the counter advances inside the update.  Not
+        # part of state_dict (the reference's keys only); .to() / .cuda() move them with the module.
+        p = next(self.parameters())
+        self.register_buffer("_m_table", momentum_table(self.pixpro_momentum, self.K).to(p.device), persistent=False)
+        self.register_buffer("_k_t", torch.zeros(1, dtype=torch.int64, device=p.device), persistent=False)
         self.k = int(args.num_instances * 1. / world_size / args.batch_size * (args.start_epoch - 1))
+
+    @property
+    def k(self) -> int:
+        """The schedule position (:231): iterations taken so far.  Reading it synchronises with the device."""
+        return int(self._k_t.item())
+
+    @k.setter
+    def k(self, value: int) -> None:
+        if value < 0:
+            raise ValueError(f"PixPro.k must be >= 0, got {value}")
+        self._k_t.fill_(int(value))
 
     def _pairs(self):
         mods = [(self.encoder_1, self.encoder_k_1), (self.encoder_2, self.encoder_k_2), (self.encoder_3, self.encoder_k_3),
@@ -89,9 +122,11 @@ class PixPro(nn.Module):
 
     @torch.no_grad()
     def _momentum_update_key_encoder(self):
-        """:258-289 -- cosine schedule, then every parameter pair in multi-tensor launches."""
-        m = 1. - (1. - self.pixpro_momentum) * (math.cos(math.pi * self.k / self.K) + 1) / 2.
-        self.k = self.k + 1
+        """:258-289 -- cosine schedule, then every parameter pair in multi-tensor launches.  The momentum pair is read
+        from the device table at the device counter, which then advances: no host read, so the update can be
+        captured in a CUDA graph and each replay takes the next step of the schedule."""
+        m = self._m_table.index_select(0, self._k_t.clamp(max=self.K)).view(2)
+        self._k_t.add_(1)
         pairs = list(self._pairs())
         soptim.momentum_update([p for p, _ in pairs], [p for _, p in pairs], m)
 
