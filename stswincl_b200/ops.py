@@ -63,6 +63,14 @@ def count_extra_launches(n: int) -> None:
         LAUNCHES += n
 
 
+MT_MAX = 48          # tensors per launch of the multi-tensor streams (MT_MAX of csrc/trainaux.cu)
+
+
+def mt_launches(n_tensors: int, per_launch: int = 1) -> int:
+    """Kernels of a multi-tensor C-ABI call over ``n_tensors`` tensors: ``per_launch`` for every MT_MAX of them."""
+    return per_launch * ((n_tensors + MT_MAX - 1) // MT_MAX)
+
+
 class _launch:
     """Context of one C-ABI call: makes the tensor's device current for the duration of the call -- on the torch side
     (``torch.cuda.device``, restored on exit, so a call on a tensor of another GPU never changes the caller's current
@@ -356,4 +364,4 @@ def gather_cast(dst, src) -> None:
                                             (ctypes.c_void_p * n)(*[s.data_ptr() for s in src]),
                                             (ctypes.c_int64 * n)(*[s.numel() for s in src]), n, int(to_bf16), _stream(dst[0]))
     _lib.check(st, "stswin_gather_cast")
-    count_extra_launches((n + 47) // 48 - 1)
+    count_extra_launches(mt_launches(n) - 1)

@@ -23,7 +23,7 @@ CUDA fp32 parameters only -- no CPU path.
 from __future__ import annotations
 
 import ctypes
-from typing import Iterable, Sequence
+from typing import Iterable, Optional, Sequence
 
 import torch
 from torch.optim.optimizer import Optimizer
@@ -53,12 +53,58 @@ def _check_f32(tensors: Iterable[torch.Tensor], what: str) -> None:
             raise StswinError(f"{what}: tensors must be contiguous fp32, got {t.dtype} (contiguous={t.is_contiguous()})")
 
 
-def _ptrs(tensors: Sequence[torch.Tensor]):
-    return (ctypes.c_void_p * len(tensors))(*[t.data_ptr() for t in tensors])
+def _ptrs(tensors: Sequence[Optional[torch.Tensor]]):
+    return (ctypes.c_void_p * len(tensors))(*[None if t is None else t.data_ptr() for t in tensors])
 
 
 def _numels(tensors: Sequence[torch.Tensor]):
     return (ctypes.c_int64 * len(tensors))(*[t.numel() for t in tensors])
+
+
+def _group_grads(param_groups, grads, who: str):
+    """List of (group, params, gradients) of every parameter group with parameters to update: those with ``p.grad``, or
+    with ``grads`` every ``requires_grad`` parameter in group order with its entry of the list.  Parameters must be
+    contiguous fp32 CUDA tensors; gradients dense contiguous CUDA tensors, all fp32 or all bf16, one per parameter and of
+    its size.  Every group is checked before the list is returned, so a refused step updates no group."""
+    if grads is not None:
+        n_req = sum(p.requires_grad for group in param_groups for p in group["params"])
+        if len(grads) != n_req:
+            raise StswinError(f"{who}: {len(grads)} gradients for {n_req} parameters that require grad")
+    out, gi = [], 0
+    for group in param_groups:
+        if grads is None:
+            params = [p for p in group["params"] if p.grad is not None]
+            gl = [p.grad for p in params]
+        else:
+            params = [p for p in group["params"] if p.requires_grad]
+            gl = list(grads[gi:gi + len(params)])
+            gi += len(params)
+        if not params:
+            continue
+        _check_f32(params, who)
+        gdt = gl[0].dtype
+        if gdt not in (torch.float32, torch.bfloat16) or any(g.dtype != gdt or g.is_sparse or not g.is_cuda or
+                                                             not g.is_contiguous() or g.numel() != p.numel()
+                                                             for g, p in zip(gl, params)):
+            raise StswinError(f"{who}: gradients must be dense contiguous CUDA tensors, all fp32 or all bf16, one per "
+                              "parameter and of its size")
+        out.append((group, params, gl))
+    return out
+
+
+def _momentum_buffers(state, params, who: str):
+    """The momentum buffers of ``params`` and the host array of first-step flags.  A parameter without one gets an
+    uninitialised buffer and the flag, on which the kernel writes buf = g to every element."""
+    _check_f32([state[p]["momentum_buffer"] for p in params if state[p].get("momentum_buffer") is not None],
+               f"{who} (momentum_buffer)")                  # before any new buffer exists
+    bufs, first = [], (ctypes.c_uint8 * len(params))()
+    for i, p in enumerate(params):
+        st = state[p]
+        if st.get("momentum_buffer") is None:
+            st["momentum_buffer"] = torch.empty_like(p, memory_format=torch.contiguous_format)
+            first[i] = 1
+        bufs.append(st["momentum_buffer"])
+    return bufs, first
 
 
 @torch.no_grad()
@@ -90,12 +136,13 @@ def momentum_update(params_q: Iterable[torch.Tensor], params_k: Iterable[torch.T
         m, om, m_dev = 0.0, 0.0, momentum.data_ptr()
     else:
         m, om, m_dev = float(momentum), float(1. - momentum), None
-    shadows = [_shadow_ptr(p, shadow) for p in pk]
+    shadows = [_shadow(p, shadow) for p in pk]
     n_bytes = sum(t.numel() for t in k) * 12 + sum(t.numel() for t, s in zip(k, shadows) if s is not None) * 2
     with ops._launch("ema_update", float(n_bytes), k[0]):                   # read k, q; write k (+ shadow)
-        st = _lib.load().stswin_ema_update(_ptrs(k), _ptrs(q), (ctypes.c_void_p * len(shadows))(*shadows), _numels(k),
-                                           len(k), m, om, m_dev, ops._stream(k[0]))
+        st = _lib.load().stswin_ema_update(_ptrs(k), _ptrs(q), _ptrs(shadows), _numels(k), len(k), m, om, m_dev,
+                                           ops._stream(k[0]))
     _lib.check(st, "stswin_ema_update")
+    ops.count_extra_launches(ops.mt_launches(len(k)) - 1)
 
 
 def _lr_arg(lr, dev, who: str):
@@ -175,46 +222,16 @@ class LARS(Optimizer):
             with torch.enable_grad():
                 loss = closure()
         lib = _lib.load()
-        if grads is not None:
-            n_req = sum(p.requires_grad for group in self.optim.param_groups for p in group['params'])
-            if len(grads) != n_req:
-                raise StswinError(f"LARS.step: {len(grads)} gradients for {n_req} parameters that require grad")
-        gi = 0
-        for group in self.optim.param_groups:
-            if grads is None:
-                params = [p for p in group['params'] if p.grad is not None]
-                gl = [p.grad for p in params]
-            else:
-                params = [p for p in group['params'] if p.requires_grad]
-                gl = list(grads[gi:gi + len(params)])
-                gi += len(params)
-            if not params:
-                continue
+        for group, params, gl in _group_grads(self.optim.param_groups, grads, "LARS.step"):
             if group.get('maximize', False):
                 raise StswinError("LARS: maximize=True is not supported")
-            _check_f32(params, "LARS.step")
             gdt = gl[0].dtype
-            if gdt not in (torch.float32, torch.bfloat16) or any(g.dtype != gdt or not g.is_contiguous() or not g.is_cuda or
-                                                                 g.numel() != p.numel() for g, p in zip(gl, params)):
-                raise StswinError("LARS.step: gradients must be contiguous CUDA tensors, all fp32 or all bf16, one per "
-                                  "parameter and of its size")
             lr, lr_dev = _lr_arg(group['lr'], params[0].device, "LARS.step")
             momentum, dampening = float(group['momentum']), float(group['dampening'])
             ignore = group.get('ignore', None)
             lars = ignore is not None and not ignore          # lars.py:125
-            bufs, first = None, None
-            if momentum != 0:
-                bufs, flags = [], []
-                for p in params:
-                    st = self.optim.state[p]
-                    buf = st.get('momentum_buffer')
-                    flags.append(1 if buf is None else 0)
-                    if buf is None:
-                        buf = st['momentum_buffer'] = torch.empty_like(p, memory_format=torch.contiguous_format)
-                    bufs.append(buf)
-                _check_f32(bufs, "LARS.step (momentum_buffer)")
-                first = (ctypes.c_uint8 * len(flags))(*flags)
-            shadows = [_shadow_ptr(p, self.shadow) for p in params]
+            bufs, first = _momentum_buffers(self.optim.state, params, "LARS.step") if momentum != 0 else (None, None)
+            shadows = [_shadow(p, self.shadow) for p in params]
             dev = params[0].device
             norms = torch.empty(2 * len(params), dtype=torch.float64, device=dev) if lars else None
             write = grads is None                                               # the p.grad contract of the reference
@@ -224,12 +241,13 @@ class LARS(Optimizer):
                 sum(p.numel() for p, s in zip(params, shadows) if s is not None) * 2
             with ops._launch("lars_sgd_step", float(n_bytes), params[0]):
                 st = lib.stswin_lars_sgd_step(_ptrs(params), _ptrs(gl), _ptrs(bufs) if bufs else None,
-                                              (ctypes.c_void_p * len(shadows))(*shadows), _numels(params), first,
+                                              _ptrs(shadows), _numels(params), first,
                                               len(params), int(gdt == torch.bfloat16), int(write), lr, lr_dev, momentum,
                                               dampening, int(bool(group['nesterov'])), float(group['weight_decay']),
                                               int(lars), float(self.trust_coef), float(self.eps),
                                               norms.data_ptr() if norms is not None else None, ops._stream(params[0]))
             _lib.check(st, "stswin_lars_sgd_step")
+            ops.count_extra_launches(ops.mt_launches(len(params), 2 if lars else 1) - 1)       # norms + update per launch
         return loss
 
 
@@ -254,12 +272,12 @@ def bf16_weight(w: torch.Tensor) -> torch.Tensor:
 
 class FusedAdam(Optimizer):
     """``torch.optim.Adam`` semantics (the optimiser of ``seg18/train_swin.py``; no amsgrad / maximize) as multi-tensor
-    launches of ``stswin_adam_step``: 32 tensors per launch, step count on the device (CUDA-graph capturable), and the
+    launches of ``stswin_adam_step``: 48 tensors per launch, step count on the device (CUDA-graph capturable), and the
     bf16 shadow of every >= 2-D weight written in the same pass (``bf16_weight``).  State keys ``exp_avg`` /
     ``exp_avg_sq`` as in torch; the step count is one device scalar per group (``group['step_t']``).
 
-    ``step(grads=...)`` takes the gradients from a list (fp32 or bf16, one per parameter with a gradient) instead of
-    ``p.grad`` -- the bf16 bucket views of a data-parallel all-reduce (``dist.SegmentedStep``)."""
+    ``step(grads=...)`` takes the gradients from a list (fp32 or bf16, one per ``requires_grad`` parameter in group
+    order) instead of ``p.grad`` -- the bf16 bucket views of a data-parallel all-reduce (``dist.SegmentedStep``)."""
 
     def __init__(self, params, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0, shadow: bool = True):
         if lr < 0 or eps < 0 or not (0 <= betas[0] < 1) or not (0 <= betas[1] < 1) or weight_decay < 0:
@@ -272,8 +290,6 @@ class FusedAdam(Optimizer):
         if not st:
             st["exp_avg"] = torch.zeros_like(p, memory_format=torch.contiguous_format)
             st["exp_avg_sq"] = torch.zeros_like(p, memory_format=torch.contiguous_format)
-            if self.shadow and p.dim() >= 2:
-                p._stswin_shadow = (p.detach().to(torch.bfloat16), p._version)
         return st
 
     @torch.no_grad()
@@ -283,45 +299,26 @@ class FusedAdam(Optimizer):
             with torch.enable_grad():
                 loss = closure()
         lib = _lib.load()
-        gi = 0
-        for group in self.param_groups:
-            if grads is None:
-                params = [p for p in group["params"] if p.grad is not None]
-                gl = [p.grad for p in params]
-            else:
-                params = [p for p in group["params"] if p.requires_grad]
-                gl = list(grads[gi:gi + len(params)])
-                gi += len(params)
-            if not params:
-                continue
-            _check_f32(params, "FusedAdam.step")
+        for group, params, gl in _group_grads(self.param_groups, grads, "FusedAdam.step"):
             gdt = gl[0].dtype
-            if gdt not in (torch.float32, torch.bfloat16) or any(g.dtype != gdt or not g.is_contiguous() or not g.is_cuda for g in gl):
-                raise StswinError("FusedAdam.step: gradients must be contiguous CUDA tensors, all fp32 or all bf16")
             states = [self._state(p) for p in params]
             if "step_t" not in group:
                 group["step_t"] = torch.zeros((), dtype=torch.float32, device=params[0].device)
-            shadows = []
-            for p in params:
-                sh = getattr(p, "_stswin_shadow", None)
-                if sh is not None and sh[1] != p._version:       # stale shadow: the kernel rewrites it anyway
-                    p._stswin_shadow = sh = (sh[0], p._version)
-                shadows.append(sh[0].data_ptr() if sh is not None else None)
+            shadows = [_shadow(p, self.shadow) for p in params]
             n_bytes = sum(p.numel() for p in params) * (28 + gl[0].element_size() - 4 + 2)
             b1, b2 = group["betas"]
             with ops._launch("adam", float(n_bytes), params[0]):
                 st = lib.stswin_adam_step(_ptrs(params), _ptrs(gl), _ptrs([s["exp_avg"] for s in states]),
-                                          _ptrs([s["exp_avg_sq"] for s in states]),
-                                          (ctypes.c_void_p * len(shadows))(*shadows), _numels(params), len(params),
+                                          _ptrs([s["exp_avg_sq"] for s in states]), _ptrs(shadows), _numels(params), len(params),
                                           int(gdt == torch.bfloat16), float(group["lr"]), float(b1), float(b2), float(group["eps"]),
                                           float(group["weight_decay"]), float(grad_scale), group["step_t"].data_ptr(),
                                           ops._stream(params[0]))
             _lib.check(st, "stswin_adam_step")
-            ops.count_extra_launches((len(params) + 31) // 32)
+            ops.count_extra_launches(ops.mt_launches(len(params)))                  # + the step-count tick
         return loss
 
 
-def _shadow_ptr(p: torch.Tensor, enabled: bool):
+def _shadow(p: torch.Tensor, enabled: bool) -> Optional[torch.Tensor]:
     """The bf16 shadow of ``p`` that an update kernel rewrites (created for >= 2-D weights when ``enabled``), or None."""
     sh = getattr(p, "_stswin_shadow", None)
     if sh is None or sh[0].device != p.device:
@@ -330,7 +327,7 @@ def _shadow_ptr(p: torch.Tensor, enabled: bool):
         sh = p._stswin_shadow = (p.detach().to(torch.bfloat16), p._version)
     elif sh[1] != p._version:                      # stale shadow: the kernel rewrites it anyway
         sh = p._stswin_shadow = (sh[0], p._version)
-    return sh[0].data_ptr()
+    return sh[0]
 
 
 class FusedSGD(Optimizer):
@@ -381,49 +378,21 @@ class FusedSGD(Optimizer):
             with torch.enable_grad():
                 loss = closure()
         lib = _lib.load()
-        gi = 0
-        for group in self.param_groups:
-            if grads is None:
-                params = [p for p in group["params"] if p.grad is not None]
-                gl = [p.grad for p in params]
-            else:
-                params = [p for p in group["params"] if p.requires_grad]
-                gl = list(grads[gi:gi + len(params)])
-                gi += len(params)
-            if not params:
-                continue
-            _check_f32(params, "FusedSGD.step")
-            if any(g.is_sparse for g in gl):
-                raise StswinError("FusedSGD.step: sparse gradients are not supported")
+        for group, params, gl in _group_grads(self.param_groups, grads, "FusedSGD.step"):
             gdt = gl[0].dtype
-            if gdt not in (torch.float32, torch.bfloat16) or any(g.dtype != gdt or not g.is_contiguous() or not g.is_cuda or
-                                                                 g.numel() != p.numel() for g, p in zip(gl, params)):
-                raise StswinError("FusedSGD.step: gradients must be contiguous CUDA tensors, all fp32 or all bf16, one per "
-                                  "parameter and of its size")
             lr, lr_dev = _lr_arg(group["lr"], params[0].device, "FusedSGD.step")
             momentum = float(group["momentum"])
-            bufs, first = None, None
-            if momentum != 0:
-                bufs, flags = [], []
-                for p in params:
-                    st = self.state[p]
-                    buf = st.get("momentum_buffer")
-                    flags.append(1 if buf is None else 0)
-                    if buf is None:
-                        buf = st["momentum_buffer"] = torch.zeros_like(p, memory_format=torch.contiguous_format)
-                    bufs.append(buf)
-                _check_f32(bufs, "FusedSGD.step (momentum_buffer)")
-                first = (ctypes.c_uint8 * len(flags))(*flags)
-            shadows = [_shadow_ptr(p, self.shadow) for p in params]
+            bufs, first = _momentum_buffers(self.state, params, "FusedSGD.step") if momentum != 0 else (None, None)
+            shadows = [_shadow(p, self.shadow) for p in params]
             n_el = sum(p.numel() for p in params)
             n_bytes = n_el * (8 + gl[0].element_size() + (8 if bufs else 0)) + \
                 sum(p.numel() for p, s in zip(params, shadows) if s is not None) * 2
             with ops._launch("sgd_step", float(n_bytes), params[0]):
                 st = lib.stswin_sgd_step(_ptrs(params), _ptrs(gl), _ptrs(bufs) if bufs else None,
-                                         (ctypes.c_void_p * len(shadows))(*shadows), _numels(params), first, len(params),
+                                         _ptrs(shadows), _numels(params), first, len(params),
                                          int(gdt == torch.bfloat16), lr, lr_dev, momentum, float(1 - group["dampening"]),
                                          int(bool(group["nesterov"])), int(bool(group["maximize"])),
                                          float(group["weight_decay"]), float(grad_scale), ops._stream(params[0]))
             _lib.check(st, "stswin_sgd_step")
-            ops.count_extra_launches((len(params) + 47) // 48 - 1)
+            ops.count_extra_launches(ops.mt_launches(len(params)) - 1)
         return loss

@@ -326,6 +326,15 @@ def test_fused_sgd_errors():
     with pytest.raises(_lib.StswinError):                                                 # lr tensor on the host
         p.grad = torch.ones(3, device="cuda")
         optim.FusedSGD([p], lr=torch.tensor(0.1)).step()
+    # grads= lists that are short, long, or hold a gradient of another size (in the second group): refused before any
+    # group is updated
+    ps = [torch.zeros(3, device="cuda", requires_grad=True), torch.zeros(5, device="cuda", requires_grad=True)]
+    o = optim.FusedSGD([dict(params=ps[:1]), dict(params=ps[1:])], lr=0.1, momentum=0.9)
+    for gl in ([torch.ones(3, device="cuda")], [torch.ones(3, device="cuda"), torch.ones(5, device="cuda")] * 2,
+               [torch.ones(3, device="cuda"), torch.ones(4, device="cuda")]):
+        with pytest.raises(_lib.StswinError, match="gradients"):
+            o.step(grads=gl)
+    assert all(not torch.any(q) for q in ps) and not o.state
     # the C ABI refuses what the constructor refuses, and momentum without buffers
     lib = _lib.load()
     ptr = (ctypes.c_void_p * 1)(p.data_ptr())

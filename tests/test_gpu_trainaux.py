@@ -232,6 +232,92 @@ def test_fused_adam_matches_torch_adam_and_keeps_the_bf16_shadow():
         assert torch.equal(so.bf16_weight(ours[0]), ours[0].detach().to(torch.bfloat16))
 
 
+def test_fused_adam_many_tensors_matches_torch_adam():
+    """80 tensors in two groups of 60 and 20 (the first takes two launches: 48, then 12), fp32 and bf16 gradients, sizes
+    around the 4096-element block size, and a 4-byte-offset view (the scalar path) in each launch of the first group."""
+    from stswincl_b200 import optim as so
+    gen = torch.Generator().manual_seed(7)
+    shapes = [(1,), (3,), (4095,), (4096,), (4097,), (100, 1000)] + [(5 + 11 * i,) for i in range(74)]
+    for gdtype in (torch.float32, torch.bfloat16):
+        ref = [torch.nn.Parameter(torch.randn(s, generator=gen)) for s in shapes]
+        ours = [torch.nn.Parameter(p.detach().clone().cuda()) for p in ref]
+        for i in (4, 52):                                                  # misaligned data pointers
+            host = torch.empty(ref[i].numel() + 1, device="cuda")
+            ours[i] = torch.nn.Parameter(host[1:].copy_(ref[i].detach()))
+        split = 60
+        o_ref = torch.optim.Adam([dict(params=ref[:split]), dict(params=ref[split:], lr=3e-3)], lr=1e-2, weight_decay=1e-2)
+        o_our = so.FusedAdam([dict(params=ours[:split]), dict(params=ours[split:], lr=3e-3)], lr=1e-2, weight_decay=1e-2)
+        for step in range(2):
+            grads = [(torch.randn(s, generator=gen) * (0.1 + step)).to(gdtype) for s in shapes]
+            for p, g in zip(ref, grads):
+                p.grad = g.float()
+            o_ref.step()
+            o_our.step(grads=[g.cuda() for g in grads])
+        torch.cuda.synchronize()
+        for p, q in zip(ref, ours):
+            assert rel_err(q.detach().cpu(), p.detach()) < 1e-5
+            assert rel_err(o_our.state[q]["exp_avg"].cpu(), o_ref.state[p]["exp_avg"]) < 1e-5
+
+
+def test_fused_adam_errors():
+    import ctypes
+    from stswincl_b200 import _lib, optim
+    ps = [torch.zeros(3, device="cuda", requires_grad=True), torch.zeros(5, device="cuda", requires_grad=True)]
+    o = optim.FusedAdam([dict(params=ps[:1]), dict(params=ps[1:])], lr=0.1)
+    # grads= lists that are short, long, or hold a gradient of another size (in the second group): refused before any
+    # group is updated
+    for gl in ([torch.ones(3, device="cuda")], [torch.ones(3, device="cuda"), torch.ones(5, device="cuda")] * 2,
+               [torch.ones(3, device="cuda"), torch.ones(4, device="cuda")]):
+        with pytest.raises(_lib.StswinError, match="gradients"):
+            o.step(grads=gl)
+    assert all(not torch.any(q) for q in ps) and not o.state
+    # a null tensor in the table: refused before the step count advances
+    lib = _lib.load()
+    p, step = torch.zeros(3, device="cuda"), torch.zeros((), device="cuda")
+    ptr, null = (ctypes.c_void_p * 1)(p.data_ptr()), (ctypes.c_void_p * 1)(None)
+    n = (ctypes.c_int64 * 1)(3)
+    stream = torch.cuda.current_stream().cuda_stream
+    assert lib.stswin_adam_step(ptr, null, ptr, ptr, None, n, 1, 0, 0.1, 0.9, 0.99, 1e-8, 0.0, 1.0, step.data_ptr(), stream) != 0
+    assert float(step) == 0.0 and not torch.any(p)
+
+
+def test_launch_counts_match_the_profiler():
+    """ops.LAUNCHES (bench.py's gpu_launches) counts every kernel of the multi-tensor calls, over 49 tensors: one more
+    than a launch takes."""
+    from torch.autograd import DeviceType
+    from torch.profiler import ProfilerActivity, profile
+    from stswincl_b200 import ops, optim
+    n = 49
+
+    def params():
+        return [torch.nn.Parameter(torch.randn(100 + 7 * i, 3, device="cuda")) for i in range(n)]
+
+    def with_grads(ps):
+        for p in ps:
+            p.grad = torch.randn_like(p)
+        return ps
+    adam = optim.FusedAdam(with_grads(params()))
+    sgd = optim.FusedSGD(with_grads(params()), lr=0.1, momentum=0.9)
+    lars = optim.LARS(torch.optim.SGD(optim.add_weight_decay(torch.nn.ParameterList(with_grads(params() + [
+        torch.nn.Parameter(torch.randn(50 + i, device="cuda")) for i in range(n)])), 1e-4), lr=0.1, momentum=0.9))
+    assert [len(g["params"]) for g in lars.param_groups] == [n, n]           # an `ignore` group and a LARS group
+    q, k = params(), params()
+    src = [torch.randn(1000 + i, device="cuda") for i in range(n)]
+    dst = [torch.empty(s.numel(), dtype=torch.bfloat16, device="cuda") for s in src]
+    calls = {"adam": adam.step, "sgd": sgd.step, "lars": lars.step, "ema": lambda: optim.momentum_update(q, k, 0.99),
+             "gather_cast": lambda: ops.gather_cast(dst, src)}
+    for name, fn in calls.items():
+        fn()                                     # optimizer state and shadows exist before the counted call
+        torch.cuda.synchronize()
+        n0 = ops.LAUNCHES
+        with profile(activities=[ProfilerActivity.CPU, ProfilerActivity.CUDA]) as prof:
+            fn()
+            torch.cuda.synchronize()
+        kernels = [e.name for e in prof.events() if e.device_type == DeviceType.CUDA and not e.is_user_annotation and
+                   not e.name.startswith(("Memset", "Memcpy"))]
+        assert ops.LAUNCHES - n0 == len(kernels), (name, ops.LAUNCHES - n0, kernels)
+
+
 def test_colsum_and_gather_cast():
     from stswincl_b200 import ops
     gen = torch.Generator().manual_seed(9)
